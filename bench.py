@@ -4,6 +4,7 @@
   python bench.py --gpus N --steps K --warmup W            # our arm (libganrev_cuda.so)
   python bench.py --impl reference --gpus N ...             # CPU arm: the oracle port on host cores
   python bench.py --config 5 ...                            # BASELINE configs[4]: 3x64x64 G/R, d=256 database, k=1024 kmeans
+  python bench.py ... --dump-outputs DIR                    # also write the last timed step's outputs as DIR/*.npy
 
 Workload (default, BASELINE.json configs[3] = north_star's target run): `--images` (default 1,000,000) generated 32x32
 grayscale faces from 100-dim N(0,1) noise IN TOTAL, sharded by image over the N ranks (STRONG scaling: 125k per GPU at
@@ -361,6 +362,33 @@ def verify(pkg, ctx, td, world, rank, geom, gb, rb, noise, attrs_host, n_local, 
     return ok, res
 
 
+DUMP_SEED, DUMP_IMAGE_BYTES = 20240, 32 << 20
+
+
+def dump_outputs(out_dir, pkg, ctx, n_local, search):
+    """--dump-outputs: what the last timed step left for its caller, as .npy files that two builds can be compared by (the
+    inputs are seeded, so the same arguments give the same inputs).  The images and recovered vectors stay on the device and
+    are 4 GB / 400 MB at the default size, so the same fixed, seeded sample of rows is written from both (at most 32 MB of
+    images); the top-k ids and scores of the in-step search (config 4) are written whole, the ids as float64 (exact below
+    2^53).  Under torchrun rank 0 writes, and its samples come from its own shard."""
+    Cc, Hh, Ww, nd = ctx.geom
+    n = min(n_local, DUMP_IMAGE_BYTES // (4 * Cc * Hh * Ww))
+    rows = np.sort(np.random.default_rng(DUMP_SEED).choice(n_local, size=n, replace=False))
+
+    def gather(which):
+        return np.concatenate([ctx.buffer_get(which, int(r), 1) for r in rows])
+
+    out = {"images_sample": gather(pkg._lib.BUF_IMAGES), "recovered_vectors_sample": gather(pkg._lib.BUF_ATTRS0)}
+    if search is not None:
+        ids, scores = search
+        out["topk_ids"] = ids.astype(np.float64)
+        out["topk_scores"] = scores
+    assert sum(a.nbytes for a in out.values()) <= 64 << 20
+    os.makedirs(out_dir, exist_ok=True)
+    for name, a in out.items():
+        np.save(os.path.join(out_dir, name + ".npy"), a)
+
+
 # ------------------------------------------------------------------------------------------------ main
 def main():
     ap = argparse.ArgumentParser()
@@ -380,7 +408,13 @@ def main():
     ap.add_argument("--no-cpu-baseline", action="store_true")
     ap.add_argument("--no-hbm-kernels", action="store_true", help="skip the L2 / kmeans / small-Q search bandwidth rooflines")
     ap.add_argument("--no-verify", action="store_true")
+    ap.add_argument("--dump-outputs", metavar="DIR", default="",
+                    help="after the timed steps, write what the last timed step computed to DIR/<name>.npy (see dump_outputs)")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and args.impl == "reference":
+        ap.error("--dump-outputs applies to the GPU arm only")
 
     global C, H, W, ND, TOPK
     if args.config == 5:
@@ -497,8 +531,10 @@ def main():
         step_resident()
     barrier()
     sampler.mark()
-    ms_res, launches, _ = timed(step_resident, args.steps)          # headline: per-kernel profiling OFF
+    ms_res, launches, last_res = timed(step_resident, args.steps)   # headline: per-kernel profiling OFF
     clocks = sampler.stop()
+    if args.dump_outputs and rank == 0:
+        dump_outputs(args.dump_outputs, pkg, ctx, N, last_res)
     # per-kernel profile: the same step, CUDA events around every launch of the library (separate pass)
     prof_steps = max(1, min(args.steps, 3))
     ctx.profile_reset()
