@@ -36,6 +36,8 @@ _SIGS = {
     "ganrev_fix_l2": (_i, [_vp, _i, _vp, _vp, _i64, _vp, _vp, _vp]),
     "ganrev_l2": (_i, [_vp, _vp, _vp, _i64, _i, _vp]),
     "ganrev_nearest_l2": (_i, [_vp, _vp, _i, _vp, _i64, _i, _vp, _vp]),
+    "ganrev_refine_l2": (_i, [_vp, _i, _vp, _vp, _i64, _i, _vp, _vp, _vp, _vp]),
+    "ganrev_debug_refine_grad": (_i, [_vp, _vp, _vp, _i64, C.c_float, _vp, _vp]),
     "ganrev_train_R_init": (_i, [_vp, _i, _i, _i, _i, _i, _i, _vp, _sz]),
     "ganrev_train_R_step": (_i, [_vp, _vp, _i, _vp, _sz, _vp, _vp]),
     "ganrev_train_R_state": (_i, [_vp, _i, _vp, _sz]),
@@ -213,6 +215,35 @@ class Context:
             xp = _ptr(np.zeros((1,), np.float32))   # any non-NULL pointer: an EMPTY explicit set, not the resident images
         self._chk(lib().ganrev_nearest_l2(self._h, _ptr(q), Q, xp, N, px, _ptr(ids), _ptr(dist)))
         return ids, dist
+
+    # ---- noise-vector refinement (new work: gradient descent through G from R's guess)
+    def refine_l2(self, slot, images, z0=None, iters=100, N=None, lr=0.01, beta1=0.9, beta2=0.999, eps=1e-8, prior=0.0, zclamp=0.0,
+                  want_attrs=True, want_fixed=True):
+        """`iters` Adam steps per image on ||G(z) - x||^2 + prior ||z||^2 from z0 (None: the resident ATTRS_slot rows), |z| <= zclamp
+        after each step if zclamp > 0.  images=None uses the resident IMAGES (then N is required).  Returns (z_final, G(z_final), l2)."""
+        Cc, H, W, nd = self.geom
+        images = _arr(images, np.float32)
+        z0 = _arr(z0, np.float32)
+        if images is not None:
+            N = images.shape[0]
+            assert images.shape[1:] == (Cc, H, W), images.shape
+        if z0 is not None:
+            assert z0.shape == (N, nd), z0.shape
+        hy = np.array([lr, beta1, beta2, eps, prior, zclamp], np.float32)
+        attrs = np.empty((N, nd), np.float32) if want_attrs else None
+        fixed = np.empty((N, Cc, H, W), np.float32) if want_fixed else None
+        l2 = np.empty((N,), np.float64)
+        self._chk(lib().ganrev_refine_l2(self._h, slot, _ptr(images), _ptr(z0), N, int(iters), _ptr(hy), _ptr(attrs), _ptr(fixed), _ptr(l2)))
+        return attrs, fixed, l2
+
+    def debug_refine_grad(self, images, z, prior=0.0):
+        """Tests: (gradient of ||G(z) - x||^2 + prior ||z||^2 [N x nd], f [N]) from one forward + backward pass of G."""
+        images, z = _arr(images, np.float32), _arr(z, np.float32)
+        N = z.shape[0]
+        grad = np.empty_like(z)
+        f = np.empty((N,), np.float64)
+        self._chk(lib().ganrev_debug_refine_grad(self._h, _ptr(images), _ptr(z), N, float(prior), _ptr(grad), _ptr(f)))
+        return grad, f
 
     # ---- R training step (train_r.lua:138-170)
     def train_R_init(self, C, H, W, nd, blob, tanh_out=False, fixer=False):

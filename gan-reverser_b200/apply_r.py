@@ -87,14 +87,25 @@ def detectAnomalies(nbImagesCalculations, nbImagesShow, threshold, images, noise
     return flags.astype(bool), 1.0 - l2, thr
 
 
+def refineAttributes(images, attributes, model_G, nbIterations, lr=0.01, prior=0.0, zclamp=0.0, slot=1):
+    """New work (the reference stops at R's single pass, apply_r.lua:152-153): starting from R's guess `attributes`, nbIterations
+    Adam steps per image on ||G(z) - x||^2 + prior ||z||^2 through G's backward pass on the GPU; |z| <= zclamp after every step when
+    zclamp > 0.  The refined vectors stay resident in ATTRS_slot (default: the fixer's), the distances for ctx.anomaly_flags(None, ..).
+    Returns (refined [N x nd], fixed = G(refined) [N x C x H x W], l2 = torch.dist per image [N])."""
+    return model_G.ctx.refine_l2(slot, np.asarray(images, np.float32), np.asarray(attributes, np.float32), iters=nbIterations,
+                                 lr=lr, prior=prior, zclamp=zclamp)
+
+
 def main(G=None, R=None, R_fixer=None, writeTo="r_results", seed=1, dimensions=(1, 32, 32), noiseDim=100,
-         noiseMethod="normal", colorSpace="y", nbImages=10000, ctx=None, write=True):
+         noiseMethod="normal", colorSpace="y", nbImages=10000, ctx=None, write=True, refine=0):
     """apply_r.lua main() (apply_r.lua:59-192) end to end.  `G` / `R` / `R_fixer` are paths of Torch7 `.net`
     checkpoints (read with t7.py, geometry from G's `opt` as at :62-79) or None for seeded random-init
     networks of `dimensions` / `noiseDim`.  Same constants as the reference: 16 variation steps, 10,000
     faces, 20 clusters x 15 iterations x 71 members, 5 needles x top-100, 52 pairs / 528 fixed faces, 1024
     anomaly distances at the 15 % quantile.  Returns a dict of everything computed; with `write`, also
-    saves the reference's JPEG files under `writeTo` (present.py)."""
+    saves the reference's JPEG files under `writeTo` (present.py).  refine > 0 (new work) also refines the fixer's vectors of the
+    first 1024 faces by that many Adam steps through G (refineAttributes) and writes fixed_refined.jpg / anomalies_refined.jpg
+    from them; refine = 0 leaves every output as it was."""
     from . import models, present
     from .models import default_context
     ctx = ctx or default_context()
@@ -142,6 +153,12 @@ def main(G=None, R=None, R_fixer=None, writeTo="r_results", seed=1, dimensions=(
     out["fixed"] = fixFaces(52, 512 + 16, images, attributesFixer, model_G)                       # :178-180
     flags, sims, thr = detectAnomalies(1024, 512 + 16, 0.15, images, noise, attributesFixer, model_G)   # :186-190
     out["anomalies"] = {"flags": flags, "similarities": sims, "anomalyBelow": thr}
+    if refine > 0:
+        nRef = max(1024, 512 + 16)
+        refined, fixed_r, l2_r = refineAttributes(images[:nRef], attributesFixer[:nRef], model_G, refine)
+        flags_r, thr_r = ctx.anomaly_flags(l2_r, 1024, 512 + 16, 0.15)
+        out["refined"] = {"attributes": refined, "fixed": fixed_r[:512 + 16], "flags": flags_r.astype(bool),
+                          "similarities": 1.0 - l2_r, "anomalyBelow": thr_r}
     if write:
         out["files"].append(present.save(os.path.join(writeTo, "variations.jpg"),
                                          present.toDisplayTensor(out["variations"], nrow=nbSteps, min=0, max=1.0)))
@@ -149,4 +166,11 @@ def main(G=None, R=None, R_fixer=None, writeTo="r_results", seed=1, dimensions=(
         out["files"] += present.saveSimilaritySearchImages(out["similar"], images, colorSpace, writeTo)
         out["files"] += present.saveFixedFaces(out["fixed"], colorSpace, writeTo)
         out["files"].append(present.saveAnomalies(images, flags, colorSpace, writeTo))
+        if refine > 0:
+            r = out["refined"]
+            n = r["fixed"].shape[0]
+            out["files"].append(present.save(os.path.join(writeTo, "fixed_refined.jpg"),
+                                             present.toDisplayTensor(r["fixed"], nrow=int(math.floor(math.sqrt(n))), min=0, max=1.0)))
+            out["files"].append(present.save(os.path.join(writeTo, "anomalies_refined.jpg"),
+                                             present.anomalyGrid(np.asarray(images)[:len(r["flags"])], r["flags"], colorSpace)))
     return out

@@ -80,6 +80,8 @@ struct ConvGemm {
     int w3_c;                  // C (1 or 3)
     float* taps;               // fp32 planes P[tap*C + co][pixel] (pixel = (n*Hout + oh)*Wout + ow), read by g_conv3_gather_kernel
     long long taps_plane;      // floats per plane
+    // MASKSUM variants (G's backward convs, refinement): bf16 tensor with exactly the output's layout; output = 2x2 sum-pool * [ref > 0]
+    const bf16* ref;
 };
 
 enum { ACT_NONE = 0, ACT_RELU = 1, ACT_ELU = 2, ACT_TANH = 3, ACT_SIGMOID = 4 };

@@ -344,7 +344,10 @@ __device__ __forceinline__ unsigned long long pack_f32x2(float lo, float hi) {
 // keeps 9*C packed (even, odd channel) fp32 sums per thread and writes them as planes P[tap*C + co][pixel] -- 36*C B per pixel
 // instead of the 256 B bf16 activation, and the separate tap-product GEMM (a full HBM round trip of that activation)
 // disappears.  The weights sit in shared memory as fp32 (16-byte broadcast loads); the activation is NOT rounded to bf16.
-template <int NT, int MT, int NDY, bool BRES, int ACT, bool POOL, bool OUT_FP32, int CG, int FUSE3 = 0>
+// MASKSUM (G's backward convs conv2^T / conv1^T, refinement): the pooled epilogue SUMS the 2x2 window (the adjoint of nearest
+// upsampling) and multiplies by [ref > 0], the stored forward activation (the ReLU mask) -- ref has the output's NHWC layout,
+// so each lane loads its 16 bytes of ref at the offset it stores to.  No shift, no activation.
+template <int NT, int MT, int NDY, bool BRES, int ACT, bool POOL, bool OUT_FP32, int CG, int FUSE3 = 0, bool MASKSUM = false>
 __global__ void __launch_bounds__(kThreads, 1)
 conv_tc_kernel(const __grid_constant__ CUtensorMap tmA, const __grid_constant__ CUtensorMap tmB,
                const __grid_constant__ CUtensorMap tmO, const __grid_constant__ ConvGemm p, const int n_items) {
@@ -575,6 +578,7 @@ conv_tc_kernel(const __grid_constant__ CUtensorMap tmA, const __grid_constant__ 
         // st.global per lane -- a window's four lanes write its 64 contiguous bytes, no shared-memory transpose
         constexpr bool kPoolDirect = GANREV_POOL_DIRECT && POOL && !OUT_FP32 && C::kChunk == 32;
         constexpr bool kStoreEarly = GANREV_STORE_EARLY && !POOL && !OUT_FP32 && ACT == ACT_ELU;
+        static_assert(!MASKSUM || (kPoolDirect && FUSE3 == 0), "MASKSUM is a mode of the direct pooled epilogue");
         if constexpr (FUSE3 != 0) {   // tap weights of the last conv -> shared memory (the store-transpose buffers are unused here)
             static_assert(NT == 128 && MT == 2 && !POOL && !OUT_FP32 && ACT == ACT_RELU && kEpiWarps == 8, "FUSE3 is G's Up+Conv 256->128");
             static_assert(kTaps * 128 * 4 <= C::kXposeBytes, "tap weights must fit in the store-transpose buffers");
@@ -819,26 +823,39 @@ conv_tc_kernel(const __grid_constant__ CUtensorMap tmA, const __grid_constant__ 
                             for (int k = 0; k < 16; ++k) {          // across w: the even lane keeps channels 0..15, the odd lane 16..31
                                 const float lo = __uint_as_float(a[k]), hi = __uint_as_float(a[16 + k]);
                                 const float recv = __shfl_xor_sync(0xffffffffu, wodd ? lo : hi, 1);
-                                m16[k] = fmaxf(wodd ? hi : lo, recv);
+                                if constexpr (MASKSUM) m16[k] = (wodd ? hi : lo) + recv;
+                                else m16[k] = fmaxf(wodd ? hi : lo, recv);
                             }
 #pragma unroll
                             for (int k = 0; k < 8; ++k) {           // across h: the even row keeps the first 8 of those, the odd row the last 8
                                 const float recv = __shfl_xor_sync(0xffffffffu, hodd ? m16[k] : m16[8 + k], BW);
-                                m8[k] = fmaxf(hodd ? m16[8 + k] : m16[k], recv);
+                                if constexpr (MASKSUM) m8[k] = (hodd ? m16[8 + k] : m16[k]) + recv;
+                                else m8[k] = fmaxf(hodd ? m16[8 + k] : m16[k], recv);
                             }
                             const int cs = (pair % kChunksPerTile) * CW + (wodd ? 16 : 0) + (hodd ? 8 : 0);
-                            const float4 s0 = *reinterpret_cast<const float4*>(ss + cs), s1 = *reinterpret_cast<const float4*>(ss + cs + 4);
-                            const float sh[8] = {s0.x, s0.y, s0.z, s0.w, s1.x, s1.y, s1.z, s1.w};
+                            if constexpr (!MASKSUM) {
+                                const float4 s0 = *reinterpret_cast<const float4*>(ss + cs), s1 = *reinterpret_cast<const float4*>(ss + cs + 4);
+                                const float sh[8] = {s0.x, s0.y, s0.z, s0.w, s1.x, s1.y, s1.z, s1.w};
 #pragma unroll
-                            for (int k = 0; k < 8; ++k) m8[k] = act_fn<ACT>(m8[k] + sh[k], p.act);   // max(a, b) + s == max(a + s, b + s)
-                            uint4 pk;
-                            pk.x = pack_bf16x2(m8[0], m8[1]); pk.y = pack_bf16x2(m8[2], m8[3]);
-                            pk.z = pack_bf16x2(m8[4], m8[5]); pk.w = pack_bf16x2(m8[6], m8[7]);
+                                for (int k = 0; k < 8; ++k) m8[k] = act_fn<ACT>(m8[k] + sh[k], p.act);   // max(a, b) + s == max(a + s, b + s)
+                            }
                             size_t po = 0;
                             bool lv = false;
 #pragma unroll
                             for (int m2 = 0; m2 < MT; ++m2)
                                 if (m2 == mt) { po = pix_off[m2]; lv = live[m2]; }
+                            if constexpr (MASKSUM) {   // a 2-term float sum is exact-commutative: every lane of a window forms the same sums
+                                const uint4 rv = lv ? __ldg(reinterpret_cast<const uint4*>(p.ref + po + cbase + cs)) : make_uint4(0u, 0u, 0u, 0u);
+                                const uint32_t rw[4] = {rv.x, rv.y, rv.z, rv.w};
+#pragma unroll
+                                for (int k = 0; k < 8; ++k) {   // bf16 > 0: sign bit clear and not +0
+                                    const uint32_t b = (rw[k >> 1] >> (16 * (k & 1))) & 0xFFFFu;
+                                    m8[k] = (b != 0u && b < 0x8000u) ? m8[k] : 0.0f;
+                                }
+                            }
+                            uint4 pk;
+                            pk.x = pack_bf16x2(m8[0], m8[1]); pk.y = pack_bf16x2(m8[2], m8[3]);
+                            pk.z = pack_bf16x2(m8[4], m8[5]); pk.w = pack_bf16x2(m8[6], m8[7]);
                             if (lv) __stcg(reinterpret_cast<uint4*>(reinterpret_cast<bf16*>(p.out) + po + cbase + cs), pk);
                         };
                         pool_store(pa, mta < MT ? mta : 0, ra);

@@ -19,6 +19,7 @@
 #include "nearest_tc.cuh"
 #include "train.cuh"
 #include "kmeans_tc.cuh"
+#include "refine.cuh"
 
 using namespace ganrev;
 
@@ -47,6 +48,15 @@ struct GModel {
     DevBuf b3;
     DevBuf w3f;                // fp32 [9][128] tap-major weights of the last conv for the fused conv2 epilogue
     bool fuse3 = false;
+    std::vector<float> blob;   // host copy of the fp32 weight blob: the refinement's backward layers are built from it on first use
+};
+// Noise-vector refinement (ganrev_refine_l2): G's backward layers and the activations one chunk keeps for them.  Built on the
+// first refine call, dropped when G is reloaded, so no other call's memory, launches or timings change.
+struct GRefine {
+    bool built = false;
+    TcLayer c2t, c1t, lint;    // conv2^T, conv1^T (MASKSUM pooled epilogue), Linear^T (fp32 out)
+    DevBuf w3t;                // fp32 [9][C][128] forward weights of the last conv for g_conv3_adjoint_kernel
+    DevBuf h0, h1, h2, y, glin, m, v, zs, dist;   // per chunk: activations, G(z), W_lin^T(s0 e0), Adam moments; z / distances (debug call)
 };
 struct RModel {
     bool loaded = false;
@@ -122,6 +132,7 @@ struct ganrev_ctx {
     std::vector<cudaEvent_t> ev_pool;
     // models
     GModel G;
+    GRefine GR;
     RModel R[2];
     // resident buffers + activation arena
     DevBuf buf[GANREV_BUF_COUNT];
@@ -445,9 +456,9 @@ static int check_geom(ganrev_ctx* ctx, int C, int H, int W, int nd) {
 // =================================================================================
 // layer launches
 // =================================================================================
-template <int NT, int MT, int NDY, bool BRES, int ACT, bool POOL, bool OUT_FP32, int CG, int FUSE3 = 0>
+template <int NT, int MT, int NDY, bool BRES, int ACT, bool POOL, bool OUT_FP32, int CG, int FUSE3 = 0, bool MASKSUM = false>
 static int launch_tc(ganrev_ctx* ctx, const TcLayer& L, const CUtensorMap& tmA, const ConvGemm& g, int n_items) {
-    auto kern = tc::conv_tc_kernel<NT, MT, NDY, BRES, ACT, POOL, OUT_FP32, CG, FUSE3>;
+    auto kern = tc::conv_tc_kernel<NT, MT, NDY, BRES, ACT, POOL, OUT_FP32, CG, FUSE3, MASKSUM>;
     static size_t attr_max_dev[kMaxDevices] = {};          // function attributes are per device
     size_t& attr_max = attr_max_dev[ctx->device];
     if (L.smem_bytes > attr_max) {
@@ -493,6 +504,13 @@ static int dispatch_tc(ganrev_ctx* ctx, const TcLayer& L, const CUtensorMap& tmA
         TC_FUSED(2, 2, 3) TC_FUSED(2, 1, 3) TC_FUSED(1, 1, 3)
 #undef TC_FUSED
         return fail(ctx, GANREV_EINVAL, "no fused tap-product variant for layer %s", L.name.c_str());
+    }
+    if (g.ref != nullptr) {  // G's backward convs (refinement): 2x2 sum-pool * [forward activation > 0]
+#define TC_MASKSUM(NDY_, CG_) \
+        if (L.NT == 128 && L.MT == 2 && L.NDY == NDY_ && !L.bres && g.pool && !g.out_fp32 && L.CG == CG_) return launch_tc<128, 2, NDY_, false, ACT_NONE, true, false, CG_, 0, true>(ctx, L, tmA, g, n_items);
+        TC_MASKSUM(3, 2) TC_MASKSUM(3, 1) TC_MASKSUM(1, 1)
+#undef TC_MASKSUM
+        return fail(ctx, GANREV_EINVAL, "no sum-pool / mask variant for layer %s", L.name.c_str());
     }
     // CTA-pair (cta_group::2) variants of the halo layers
     TC_CASE_CG(256, 1, 1, false, ACT_RELU, false, false, 2)   // G Up+Conv 512->256
@@ -597,6 +615,11 @@ static int run_layer(ganrev_ctx* ctx, TcLayer& L, const void* in, void* out, int
 // model loading
 // =================================================================================
 static void release_layer(TcLayer& L) { release(L.w); release(L.shift); }
+static void release_refine(GRefine& R) {
+    for (TcLayer* L : {&R.c2t, &R.c1t, &R.lint}) release_layer(*L);
+    for (DevBuf* b : {&R.w3t, &R.h0, &R.h1, &R.h2, &R.y, &R.glin, &R.m, &R.v, &R.zs, &R.dist}) release(*b);
+    R.built = false;
+}
 
 // One geometry per context: G, R and R_fixer of apply_r.lua share {C, H, W, noiseDim} (apply_r.lua:65-79), and the resident
 // buffers are sized by it.  Loading a model of a DIFFERENT geometry therefore unloads the models of the old one and empties
@@ -620,6 +643,8 @@ static int load_G_impl(ganrev_ctx* ctx, int C, int H, int W, int nd, const float
     adopt_geometry(ctx, C, H, W, nd);
     GModel& G = ctx->G;
     G.loaded = false;
+    release_refine(ctx->GR);
+    G.blob.assign(blob, blob + n_floats);
     const float* p = blob;
     const float* lw = p; p += static_cast<size_t>(F) * nd;
     const float* lb = p; p += F;
@@ -951,6 +976,158 @@ static int l2_dev(ganrev_ctx* ctx, const float* a, const float* b, int64_t N, in
     return GANREV_OK;
 }
 
+
+// ---------------------------------------------------------------- noise-vector refinement (DESIGN.md section 4.5)
+// G's backward layers, from the host copy of the blob.  With BN folded (s = scale): conv^T is a plain 3x3 conv at the high
+// resolution with weights W^T[ci][2-ky][2-kx][co] * s[co]; the 2x2 sum-pool (adjoint of nearest upsampling) and the ReLU mask of
+// the stored forward activation are the MASKSUM epilogue; Linear^T is the K = F GEMM in the forward's NHWC feature order with s0
+// folded.  N = 128 tiles: a 256-wide tile with halo reuse needs 116 KB per pipeline unit, two stages do not fit in shared memory.
+static int build_refine(ganrev_ctx* ctx) {
+    GRefine& R = ctx->GR;
+    if (R.built) return GANREV_OK;
+    const GModel& G = ctx->G;
+    const int C = G.C, H = G.H, W = G.W, nd = G.nd, HW0 = (H / 4) * (W / 4), F = G.F;
+    const float* p = G.blob.data();
+    const float* lw = p; p += static_cast<size_t>(F) * nd;
+    p += F;                                                                  // Linear bias (in the forward's shift only)
+    const float *g0 = p, *v0 = p + 3 * static_cast<size_t>(F); p += 4 * static_cast<size_t>(F);
+    const float* w1 = p; p += 256u * 512 * 9 + 256;
+    const float *g1 = p, *v1 = p + 768; p += 1024;
+    const float* w2 = p; p += 128u * 256 * 9 + 128;
+    const float *g2 = p, *v2 = p + 384; p += 512;
+    const float* w3 = p;
+    auto sc = [](const float* g, const float* v, size_t i) { return g[i] / std::sqrt(v[i] + 1e-5f); };   // fold_bn's scale
+    const int pairs = (ctx->cta_pairs & 16) ? 2 : 1;   // the pooled 128-wide tile of R conv6 (same kernel shape)
+    auto conv_t = [&](TcLayer& L, const char* name, const float* w, const float* g, const float* v, int co_f, int ci_f, int Hin, int Win) {
+        // forward conv ci_f -> co_f; adjoint co_f -> ci_f at the forward conv's (high) resolution, pooled to the forward input's
+        std::vector<float> wt(static_cast<size_t>(ci_f) * co_f * 9);
+        for (int b = 0; b < co_f; ++b) {
+            const float s = sc(g, v, b);
+            for (int a = 0; a < ci_f; ++a)
+                for (int t = 0; t < 9; ++t) wt[(static_cast<size_t>(a) * co_f + b) * 9 + t] = w[(static_cast<size_t>(b) * ci_f + a) * 9 + (8 - t)] * s;
+        }
+        BnFold one;
+        one.scale.assign(ci_f, 1.0f); one.shift.assign(ci_f, 0.0f);
+        const LayerDef d{name, KIND_CONV3, 128, 2, pairs, false, Hin, Win, co_f, ci_f, ci_f / 128, Hin / 2, Win / 2, ci_f, 1, ACT_NONE, 1.0f, 0, false};
+        return build_tc_layer(ctx, L, d, wt.data(), one);
+    };
+    RC_TRY(conv_t(R.c2t, "g_bwd_conv2", w2, g2, v2, 128, 256, H, W));
+    RC_TRY(conv_t(R.c1t, "g_bwd_conv1", w1, g1, v1, 256, 512, H / 2, W / 2));
+    {   // Linear^T: [nd (padded)][F], column fn = s*512 + c (NHWC) <- forward row fo = c*HW0 + s (View(512, sH, sW))
+        const int NT = nd <= 32 ? 32 : (nd <= 64 ? 64 : (nd <= 128 ? 128 : 256));
+        const int n_tiles = (nd + NT - 1) / NT, cp = n_tiles * NT;
+        std::vector<float> wm(static_cast<size_t>(cp) * F, 0.0f);
+        for (int c = 0; c < 512; ++c)
+            for (int s = 0; s < HW0; ++s) {
+                const size_t fo = static_cast<size_t>(c) * HW0 + s, fn = static_cast<size_t>(s) * 512 + c;
+                const float s0 = sc(g0, v0, fo);
+                for (int k = 0; k < nd; ++k) wm[static_cast<size_t>(k) * F + fn] = lw[fo * nd + k] * s0;
+            }
+        BnFold bn;
+        bn.scale.assign(cp, 0.0f); bn.shift.assign(cp, 0.0f);
+        for (int i = 0; i < nd; ++i) bn.scale[i] = 1.0f;
+        const LayerDef d{"g_bwd_linear", KIND_LINEAR, NT, 1, 1, false, 1, 1, F, nd, n_tiles, 1, 1, nd, 0, ACT_NONE, 1.0f, 1, false};
+        RC_TRY(build_tc_layer(ctx, R.lint, d, wm.data(), bn));
+    }
+    std::vector<float> w3t(static_cast<size_t>(9) * C * 128);
+    for (int t = 0; t < 9; ++t)
+        for (int co = 0; co < C; ++co)
+            for (int ci = 0; ci < 128; ++ci) w3t[(static_cast<size_t>(t) * C + co) * 128 + ci] = w3[(static_cast<size_t>(co) * 128 + ci) * 9 + t];
+    RC_TRY(upload(ctx, R.w3t, w3t.data(), w3t.size() * 4));
+    R.built = true;
+    return GANREV_OK;
+}
+
+static int refine_buffers(ganrev_ctx* ctx, int64_t CH) {
+    const GModel& G = ctx->G;
+    GRefine& R = ctx->GR;
+    const size_t px = static_cast<size_t>(G.H) * G.W;
+    RC_TRY(ensure_arena(ctx, px * 128 * 2, CH));   // e2 (the largest gradient), then e0; e1 and the last conv's tap planes in the other
+    RC_TRY(ensure(ctx, ctx->noise_bf16, static_cast<size_t>(CH) * G.kpad * 2));
+    RC_TRY(ensure(ctx, R.h0, static_cast<size_t>(CH) * G.F * 2));
+    RC_TRY(ensure(ctx, R.h1, static_cast<size_t>(CH) * px / 4 * 256 * 2));
+    RC_TRY(ensure(ctx, R.h2, static_cast<size_t>(CH) * px * 128 * 2));
+    RC_TRY(ensure(ctx, R.y, static_cast<size_t>(CH) * G.C * px * 4));
+    for (DevBuf* b : {&R.glin, &R.m, &R.v}) RC_TRY(ensure(ctx, *b, static_cast<size_t>(CH) * G.nd * 4));
+    return GANREV_OK;
+}
+
+// One forward pass of G keeping h0 / h1 / h2 (bf16 NHWC) and y = G(z) (fp32 NCHW, in R.y), then the backward pass down to
+// R.glin[n x nd] = W_lin^T (s0 e0), the gradient of ||G(z) - x||^2 without the prior term.  n <= CH images.
+static int refine_grad_chunk(ganrev_ctx* ctx, const float* d_z, const float* d_x, int n, int64_t CH) {
+    GModel& G = ctx->G;
+    GRefine& R = ctx->GR;
+    const int H = G.H, W = G.W;
+    const long long npix = static_cast<long long>(n) * H * W, plane = static_cast<long long>(CH) * H * W;
+    {
+        ProfScope ps(ctx, "g_noise_to_bf16", 0.0, static_cast<double>(n) * (G.nd * 4.0 + G.kpad * 2.0));
+        const long long tot = static_cast<long long>(n) * G.kpad;
+        noise_to_bf16_kernel<<<static_cast<unsigned>((tot + 255) / 256), 256, 0, ctx->stream>>>(d_z, G.nd, G.kpad, reinterpret_cast<bf16*>(ctx->noise_bf16.p), n);
+        CU_TRY(cudaGetLastError());
+    }
+    RC_TRY(run_layer(ctx, G.lin, ctx->noise_bf16.p, R.h0.p, n, CH));
+    RC_TRY(run_layer(ctx, G.c1, R.h0.p, R.h1.p, n, CH));
+    G.c2.g.w3 = nullptr;                                                        // unfused: h2 itself is needed
+    RC_TRY(run_layer(ctx, G.c2, R.h1.p, R.h2.p, n, CH));
+    G.c3.g.out_sN = 1; G.c3.g.out_sP = 1; G.c3.g.out_sC = static_cast<int>(plane);
+    G.c3.bytes_per_img = 2.0 * 128 + 4.0 * 9 * G.C;
+    RC_TRY(run_layer(ctx, G.c3, R.h2.p, ctx->arena[1].p, static_cast<int>(npix), CH * H * W));
+    float* y = static_cast<float*>(R.y.p);
+    {
+        ProfScope ps(ctx, "g_conv3_gather", 9.0 * npix * G.C, npix * (4.0 * 9 * G.C + 4.0 * G.C));
+        const unsigned blocks = static_cast<unsigned>((npix / 4 + 255) / 256);
+        const float* planes = static_cast<const float*>(ctx->arena[1].p);
+        if (G.C == 1) g_conv3_gather_kernel<1><<<blocks, 256, 0, ctx->stream>>>(planes, plane, static_cast<const float*>(G.b3.p), y, H, W, ilog2(H), ilog2(W), n);
+        else          g_conv3_gather_kernel<3><<<blocks, 256, 0, ctx->stream>>>(planes, plane, static_cast<const float*>(G.b3.p), y, H, W, ilog2(H), ilog2(W), n);
+        CU_TRY(cudaGetLastError());
+    }
+    bf16* e2 = static_cast<bf16*>(ctx->arena[0].p);
+    {   // per pixel: 9*C taps into 128 channels; reads y, x (9*C neighbours, cached) and h2, writes e2
+        ProfScope ps(ctx, "g_bwd_conv3", 2.0 * npix * 9 * G.C * 128, npix * (2.0 * 4 * G.C + 2.0 * 128 + 2.0 * 128));
+        const unsigned blocks = static_cast<unsigned>((npix * 16 + 255) / 256);
+        const bf16* h2 = static_cast<const bf16*>(R.h2.p);
+        const float* w3t = static_cast<const float*>(R.w3t.p);
+        if (G.C == 1) g_conv3_adjoint_kernel<1><<<blocks, 256, 0, ctx->stream>>>(y, d_x, w3t, h2, e2, H, W, ilog2(H), ilog2(W), n);
+        else          g_conv3_adjoint_kernel<3><<<blocks, 256, 0, ctx->stream>>>(y, d_x, w3t, h2, e2, H, W, ilog2(H), ilog2(W), n);
+        CU_TRY(cudaGetLastError());
+    }
+    R.c2t.g.ref = static_cast<const bf16*>(R.h1.p);
+    RC_TRY(run_layer(ctx, R.c2t, e2, ctx->arena[1].p, n, CH));                  // e1 = [h1 > 0] * sumpool(conv2^T(e2))
+    R.c1t.g.ref = static_cast<const bf16*>(R.h0.p);
+    RC_TRY(run_layer(ctx, R.c1t, ctx->arena[1].p, ctx->arena[0].p, n, CH));     // e0 = [h0 > 0] * sumpool(conv1^T(e1))
+    RC_TRY(run_layer(ctx, R.lint, ctx->arena[0].p, R.glin.p, n, CH));           // W_lin^T (s0 e0)
+    return GANREV_OK;
+}
+
+// `iters` Adam steps on every row of d_z [N x nd] (in place).  Chunks run one after another, all iterations of a chunk at a time:
+// nothing mixes images, so results do not depend on the chunk size or on which images share a call.
+static int refine_dev(ganrev_ctx* ctx, const float* d_x, float* d_z, int64_t N, int iters, const float* hyper6) {
+    GModel& G = ctx->G;
+    GRefine& R = ctx->GR;
+    const int64_t CH = std::min<int64_t>(chunk_for(ctx, G.H, G.W), std::max<int64_t>(N, 1));
+    RC_TRY(build_refine(ctx));
+    RC_TRY(refine_buffers(ctx, CH));
+    const long long px = static_cast<long long>(G.C) * G.H * G.W;
+    for (int64_t n0 = 0; n0 < N; n0 += CH) {
+        const int n = static_cast<int>(std::min<int64_t>(CH, N - n0));
+        const long long ne = static_cast<long long>(n) * G.nd;
+        float* z = d_z + n0 * G.nd;
+        CU_TRY(cudaMemsetAsync(R.m.p, 0, sizeof(float) * ne, ctx->stream));
+        CU_TRY(cudaMemsetAsync(R.v.p, 0, sizeof(float) * ne, ctx->stream));
+        for (int t = 1; t <= iters; ++t) {
+            RC_TRY(refine_grad_chunk(ctx, z, d_x + n0 * px, n, CH));
+            RefineHyper h{};
+            h.beta1 = hyper6[1]; h.beta2 = hyper6[2]; h.eps = hyper6[3]; h.prior2 = 2.0f * hyper6[4]; h.zclamp = hyper6[5];
+            h.step_size = static_cast<float>(static_cast<double>(hyper6[0]) * std::sqrt(1.0 - std::pow(static_cast<double>(h.beta2), static_cast<double>(t))) /
+                                             (1.0 - std::pow(static_cast<double>(h.beta1), static_cast<double>(t))));
+            ProfScope ps(ctx, "refine_adam", 12.0 * ne, 24.0 * ne);
+            refine_adam_kernel<<<static_cast<unsigned>((ne + 255) / 256), 256, 0, ctx->stream>>>(z, static_cast<const float*>(R.glin.p), static_cast<float*>(R.m.p), static_cast<float*>(R.v.p), ne, h);
+            CU_TRY(cudaGetLastError());
+        }
+    }
+    return GANREV_OK;
+}
+
 // =================================================================================
 // C ABI
 // =================================================================================
@@ -999,6 +1176,7 @@ void ganrev_destroy(ganrev_ctx* ctx) {
     for (TcLayer* L : {&ctx->G.lin, &ctx->G.c1, &ctx->G.c2, &ctx->G.c3}) release_layer(*L);
     release(ctx->G.b3);
     release(ctx->G.w3f);
+    release_refine(ctx->GR);
     for (int s = 0; s < 2; ++s) {
         RModel& R = ctx->R[s];
         release(R.c1pack); release(R.c1w); release(R.c1shift);
@@ -1228,6 +1406,89 @@ int ganrev_l2(ganrev_ctx* ctx, const float* a, const float* b, int64_t N, int px
     ctx->l2_valid = N;
     CU_TRY(cudaMemcpyAsync(l2, ctx->l2buf.p, sizeof(double) * N, cudaMemcpyDeviceToHost, ctx->stream));
     return finish(ctx);
+}
+
+
+static int refine_check(ganrev_ctx* ctx) {
+    if (!ctx->G.loaded) return fail(ctx, GANREV_ESTATE, "G not loaded");
+    if (ctx->conv_impl != 0) return fail(ctx, GANREV_EINVAL, "refinement runs on the tcgen05 kernels only (conv_impl 0)");
+    return GANREV_OK;
+}
+
+int ganrev_refine_l2(ganrev_ctx* ctx, int slot, const float* images, const float* z0, int64_t N, int iters, const float* hyper6,
+                     float* attrs, float* fixed, double* l2) {
+    if (!ctx || N < 0 || slot < 0 || slot > 1 || !hyper6) return ctx ? fail(ctx, GANREV_EINVAL, "bad refine_l2 arguments") : GANREV_EINVAL;
+    if (iters < 0 || !(hyper6[0] > 0.0f) || !(hyper6[4] >= 0.0f))
+        return fail(ctx, GANREV_EINVAL, "refine_l2 needs iters >= 0, lr > 0, prior >= 0 (got %d, %g, %g)", iters, hyper6[0], hyper6[4]);
+    RC_TRY(refine_check(ctx));
+    if (N == 0) return GANREV_OK;
+    CU_TRY(cudaSetDevice(ctx->device));
+    RC_TRY(stage_input(ctx, GANREV_BUF_IMAGES, images, N));
+    const int ob = slot == 0 ? GANREV_BUF_ATTRS0 : GANREV_BUF_ATTRS1;
+    if (z0) {
+        RC_TRY(stage_input(ctx, ob, z0, N));                  // (un-sets a database aliasing ATTRS0)
+    } else {
+        if (ctx->buf_rows[ob] < N || !ctx->buf[ob].p)
+            return fail(ctx, GANREV_ESTATE, "resident buffer %d holds %lld rows, need %lld", ob, (long long)ctx->buf_rows[ob], (long long)N);
+        buf_touch(ctx, ob);                                    // refined in place
+    }
+    RC_TRY(buf_reserve(ctx, GANREV_BUF_FIXED, N));
+    ctx->l2_valid = 0;
+    RC_TRY(ensure(ctx, ctx->l2buf, sizeof(double) * static_cast<size_t>(N)));
+    const float* d_img = static_cast<const float*>(ctx->buf[GANREV_BUF_IMAGES].p);
+    float* d_att = static_cast<float*>(ctx->buf[ob].p);
+    float* d_fix = static_cast<float*>(ctx->buf[GANREV_BUF_FIXED].p);
+    if (iters > 0) RC_TRY(refine_dev(ctx, d_img, d_att, N, iters, hyper6));
+    // fixed / l2 from the same path as ganrev_fix_l2: bit-identical to ganrev_forward_G(z_final) + ganrev_l2
+    RC_TRY(forward_G_dev(ctx, d_att, N, d_fix));
+    ctx->buf_rows[GANREV_BUF_FIXED] = N;
+    RC_TRY(l2_dev(ctx, d_img, d_fix, N, ctx->G.C * ctx->G.H * ctx->G.W, static_cast<double*>(ctx->l2buf.p)));
+    ctx->l2_valid = N;
+    RC_TRY(fetch_output(ctx, ob, attrs, N));
+    RC_TRY(fetch_output(ctx, GANREV_BUF_FIXED, fixed, N));
+    if (l2) CU_TRY(cudaMemcpyAsync(l2, ctx->l2buf.p, sizeof(double) * N, cudaMemcpyDeviceToHost, ctx->stream));
+    return finish(ctx);
+}
+
+int ganrev_debug_refine_grad(ganrev_ctx* ctx, const float* images, const float* z, int64_t N, float prior, float* grad, double* f) {
+    if (!ctx || !images || !z || !grad || !f || N < 0 || !(prior >= 0.0f)) return ctx ? fail(ctx, GANREV_EINVAL, "bad debug_refine_grad arguments") : GANREV_EINVAL;
+    RC_TRY(refine_check(ctx));
+    if (N == 0) return GANREV_OK;
+    CU_TRY(cudaSetDevice(ctx->device));
+    const GModel& G = ctx->G;
+    GRefine& R = ctx->GR;
+    const int64_t CH = std::min<int64_t>(chunk_for(ctx, G.H, G.W), N);
+    const long long px = static_cast<long long>(G.C) * G.H * G.W, nz = N * G.nd;
+    RC_TRY(build_refine(ctx));
+    RC_TRY(refine_buffers(ctx, CH));
+    RC_TRY(ensure(ctx, ctx->stage_a, sizeof(float) * N * px));
+    RC_TRY(ensure(ctx, ctx->stage_b, sizeof(float) * nz));
+    RC_TRY(ensure(ctx, R.zs, sizeof(float) * nz));
+    RC_TRY(ensure(ctx, R.dist, sizeof(double) * N));
+    const float* d_x = static_cast<const float*>(ctx->stage_a.p);
+    const float* d_z = static_cast<const float*>(R.zs.p);
+    float* d_g = static_cast<float*>(ctx->stage_b.p);
+    double* d_dist = static_cast<double*>(R.dist.p);
+    CU_TRY(cudaMemcpyAsync(ctx->stage_a.p, images, sizeof(float) * N * px, cudaMemcpyHostToDevice, ctx->stream));
+    CU_TRY(cudaMemcpyAsync(R.zs.p, z, sizeof(float) * nz, cudaMemcpyHostToDevice, ctx->stream));
+    for (int64_t n0 = 0; n0 < N; n0 += CH) {
+        const int n = static_cast<int>(std::min<int64_t>(CH, N - n0));
+        const long long ne = static_cast<long long>(n) * G.nd;
+        RC_TRY(refine_grad_chunk(ctx, d_z + n0 * G.nd, d_x + n0 * px, n, CH));
+        refine_grad_kernel<<<static_cast<unsigned>((ne + 255) / 256), 256, 0, ctx->stream>>>(static_cast<const float*>(R.glin.p), d_z + n0 * G.nd, 2.0f * prior, d_g + n0 * G.nd, ne);
+        CU_TRY(cudaGetLastError());
+        RC_TRY(l2_dev(ctx, d_x + n0 * px, static_cast<const float*>(R.y.p), n, static_cast<int>(px), d_dist + n0));
+    }
+    std::vector<double> dist(N);
+    CU_TRY(cudaMemcpyAsync(grad, d_g, sizeof(float) * nz, cudaMemcpyDeviceToHost, ctx->stream));
+    CU_TRY(cudaMemcpyAsync(dist.data(), d_dist, sizeof(double) * N, cudaMemcpyDeviceToHost, ctx->stream));
+    RC_TRY(finish(ctx));
+    for (int64_t i = 0; i < N; ++i) {   // f = ||G(z) - x||^2 + prior ||z||^2
+        double zz = 0.0;
+        for (int k = 0; k < G.nd; ++k) zz += static_cast<double>(z[i * G.nd + k]) * z[i * G.nd + k];
+        f[i] = dist[i] * dist[i] + static_cast<double>(prior) * zz;
+    }
+    return GANREV_OK;
 }
 
 }  // extern "C"

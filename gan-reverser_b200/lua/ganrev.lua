@@ -42,6 +42,7 @@ int ganrev_search_rows(ganrev_ctx* ctx, const int64_t* rows, int Q, int k, int64
 int ganrev_kmeans(ganrev_ctx* ctx, int k, int niter, const float* init_centroids, float* centroids, float* total_counts, int32_t* last_labels);
 int ganrev_assign_cosine_min(ganrev_ctx* ctx, const float* centroids, int k, int32_t* cluster, float* cosv);
 int ganrev_cluster_members(ganrev_ctx* ctx, int k, int m, const float* images, int px, int64_t* member_ids, int32_t* member_counts, float* mean_images);
+int ganrev_refine_l2(ganrev_ctx* ctx, int slot, const float* images, const float* z0, int64_t N, int iters, const float* hyper6, float* attrs, float* fixed, double* l2);
 int ganrev_train_R_init(ganrev_ctx* ctx, int C, int H, int W, int noise_dim, int tanh_out, int fixer, const float* blob, size_t n_floats);
 int ganrev_train_R_step(ganrev_ctx* ctx, const float* noise, int B, const uint8_t* masks, size_t mask_bytes, const float* hyper7, double* loss2);
 int ganrev_train_R_state(ganrev_ctx* ctx, int what, float* out, size_t n_floats);
@@ -288,6 +289,21 @@ function M.anomalies(ctx, images, fixed, nbImagesCalculations, nbImagesShow, thr
     local flags, thr = torch.ByteTensor(nbImagesShow), ffi.new('double[1]')
     check(ctx, lib.ganrev_anomaly_flags(ctx, l2:data(), n, nbImagesShow, threshold, flags:data(), thr))
     return flags, l2:mul(-1):add(1), tonumber(thr[0])
+end
+
+-- New work (the reference stops at R's single pass, apply_r.lua:152-153): refine recovered vectors by gradient descent through G.
+-- images = N x C x H x W, attributes = N x noiseDim (R's or R_fixer's output, the starting point), nbIterations Adam steps on
+-- ||G(z) - x||^2 + prior ||z||^2 per image; opt = {lr, beta1, beta2, eps, prior, zclamp} (defaults 0.01, 0.9, 0.999, 1e-8, 0, 0 = no
+-- clamp).  slot = which ATTRS buffer keeps the result (default 1, the fixer's).  Returns refined attributes, G(refined), distances.
+function M.refine_l2(ctx, images, attributes, nbIterations, opt, slot)
+    opt = opt or {}
+    images, attributes = images:float():contiguous(), attributes:float():contiguous()
+    local N = images:size(1)
+    local hyper = torch.FloatTensor({opt.lr or 0.01, opt.beta1 or 0.9, opt.beta2 or 0.999, opt.eps or 1e-8, opt.prior or 0, opt.zclamp or 0})
+    local refined, fixed, l2 = torch.FloatTensor(N, attributes:size(2)), torch.FloatTensor(images:size()), torch.DoubleTensor(N)
+    check(ctx, lib.ganrev_refine_l2(ctx, slot or 1, images:data(), attributes:data(), N, nbIterations, hyper:data(),
+                                    refined:data(), fixed:data(), l2:data()))
+    return refined, fixed, l2
 end
 
 -- findClosestNeighboursOf  sample.lua:128-148: images = list of image tensors, trainingSet = N x C x H x W tensor.

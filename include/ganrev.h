@@ -32,6 +32,9 @@
  *   R (models.lua:409-451): 6 x (Conv, BN) with channels C->64->64->64->128->128->128,
  *                           Linear(128*H/4*W/4 -> 512), BN, Linear(512 -> nd).
  *
+ * New work beyond the reference is marked as such: multi-GPU sharding and the refinement of recovered noise
+ * vectors by gradient descent through G (ganrev_refine_l2).
+ *
  * One geometry per context: G, R and R_fixer of apply_r.lua share {C, H, W, noiseDim}
  * (apply_r.lua:65-79) and the resident buffers are sized by it.  Loading a model with a
  * DIFFERENT geometry unloads the models of the old geometry and empties every resident
@@ -115,7 +118,7 @@ int ganrev_nearest_l2(ganrev_ctx* ctx, const float* queries, int Q, const float*
                       int64_t* ids, double* dist);
 /* apply_r.lua:370-378: sims = 1 - l2; thr = ascending sims[floor(n_calc*quantile)] (1-based);
  * flags[i] = sims[i] <= thr, i < n_show.  thr may be NULL.  l2 == NULL reuses the distances the last ganrev_fix_l2 /
- * ganrev_l2 call left on the device (GANREV_ESTATE if it left fewer than n_calc).  After ganrev_comm_init l2 / n_calc /
+ * ganrev_refine_l2 / ganrev_l2 call left on the device (GANREV_ESTATE if it left fewer than n_calc).  After ganrev_comm_init l2 / n_calc /
  * n_show describe this rank's shard (n_calc may be 0): the order statistic is taken over all ranks' n_calc values by a
  * device radix select with one 256-bin allreduce per pass; flags are this rank's first n_show. */
 int ganrev_anomaly_flags(ganrev_ctx* ctx, const double* l2, int64_t n_calc, int64_t n_show,
@@ -175,6 +178,23 @@ int ganrev_cluster_members(ganrev_ctx* ctx, int k, int m, const float* images, i
 int ganrev_train_R_init(ganrev_ctx* ctx, int C, int H, int W, int noise_dim, int tanh_out, int fixer, const float* blob, size_t n_floats);
 int ganrev_train_R_step(ganrev_ctx* ctx, const float* noise, int B, const uint8_t* masks, size_t mask_bytes, const float* hyper7, double* loss2);
 int ganrev_train_R_state(ganrev_ctx* ctx, int what, float* out, size_t n_floats);
+
+/* ---- noise-vector refinement (new work; the reference stops at R's single pass, apply_r.lua:152-153) --------------
+ * For each image x_i, `iters` steps of Adam (optim.adam's update, as ganrev_train_R_step applies it) on
+ *   f(z) = ||G(z) - x_i||^2 + prior * ||z||^2,  then, if zclamp > 0, |z| <= zclamp elementwise after every step.
+ * hyper6 = {lr, beta1, beta2, eps, prior, zclamp}.  images NULL = resident IMAGES; z0 NULL = the first N rows of resident
+ * ATTRS_slot (GANREV_ESTATE if it holds fewer).  The refined vectors are left in ATTRS_slot (slot 0: un-sets an aliasing
+ * database, as ganrev_fix_l2 does), G(z_final) in FIXED, and l2[i] = torch.dist(x_i, G(z_final)) stays on the device for
+ * ganrev_anomaly_flags(l2 = NULL); fixed and l2 are exactly ganrev_forward_G(z_final) + ganrev_l2, and iters = 0 is the fix
+ * path applied to z0.  attrs / fixed / l2 may be NULL.  GANREV_EINVAL for iters < 0, lr <= 0 or prior < 0.  Deterministic,
+ * independent of the chunk size and of which other images share the call.  The gradient is G's backward pass on the tensor
+ * cores, built on the first call (not at ganrev_load_G).  Image-sharded: after ganrev_comm_init every rank refines its own
+ * rows, and the call makes no collective. */
+int ganrev_refine_l2(ganrev_ctx* ctx, int slot, const float* images, const float* z0, int64_t N, int iters,
+                     const float* hyper6, float* attrs, float* fixed, double* l2);
+/* Tests: grad [N x nd] = the gradient of f at z and f [N], one forward + backward (no optimiser step). */
+int ganrev_debug_refine_grad(ganrev_ctx* ctx, const float* images, const float* z, int64_t N, float prior,
+                             float* grad, double* f);
 
 /* ---- measurement hooks (bench.py) ----------------------------------------------- */
 void*    ganrev_stream(ganrev_ctx* ctx);                 /* cudaStream_t all work runs on */
