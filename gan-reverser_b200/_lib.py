@@ -38,6 +38,7 @@ _SIGS = {
     "ganrev_nearest_l2": (_i, [_vp, _vp, _i, _vp, _i64, _i, _vp, _vp]),
     "ganrev_refine_l2": (_i, [_vp, _i, _vp, _vp, _i64, _i, _vp, _vp, _vp, _vp]),
     "ganrev_debug_refine_grad": (_i, [_vp, _vp, _vp, _i64, C.c_float, _vp, _vp]),
+    "ganrev_debug_refine_stage": (_i, [_vp, _vp, _vp, _i64, _i, _vp, _sz]),
     "ganrev_train_R_init": (_i, [_vp, _i, _i, _i, _i, _i, _i, _vp, _sz]),
     "ganrev_train_R_step": (_i, [_vp, _vp, _i, _vp, _sz, _vp, _vp]),
     "ganrev_train_R_state": (_i, [_vp, _i, _vp, _sz]),
@@ -244,6 +245,23 @@ class Context:
         f = np.empty((N,), np.float64)
         self._chk(lib().ganrev_debug_refine_grad(self._h, _ptr(images), _ptr(z), N, float(prior), _ptr(grad), _ptr(f)))
         return grad, f
+
+    REFINE_STAGES = ("h0", "h1", "h2", "y", "e2", "e1", "e0", "glin")
+
+    def debug_refine_stage(self, images, z, stage):
+        """Tests: the buffer of one stage of refine_l2's forward + backward pass of G (ganrev.h), rows in input order.  bf16 stages
+        come back as their uint16 bits, NHWC; y is float32 NCHW, glin float32 [N x nd].  `stage` is an index or a name."""
+        Cc, H, W, nd = self.geom
+        s = self.REFINE_STAGES.index(stage) if isinstance(stage, str) else int(stage)
+        images, z = _arr(images, np.float32), _arr(z, np.float32)
+        N = z.shape[0]
+        shapes = {0: ((H // 4, W // 4, 512), np.uint16), 1: ((H // 2, W // 2, 256), np.uint16), 2: ((H, W, 128), np.uint16),
+                  3: ((Cc, H, W), np.float32), 4: ((H, W, 128), np.uint16), 5: ((H // 2, W // 2, 256), np.uint16),
+                  6: ((H // 4, W // 4, 512), np.uint16), 7: ((nd,), np.float32)}
+        shape, dt = shapes.get(s, ((1,), np.uint8))
+        out = np.empty((N,) + shape, dt)
+        self._chk(lib().ganrev_debug_refine_stage(self._h, _ptr(images), _ptr(z), N, s, _ptr(out), out.nbytes))
+        return out
 
     # ---- R training step (train_r.lua:138-170)
     def train_R_init(self, C, H, W, nd, blob, tanh_out=False, fixer=False):

@@ -48,6 +48,7 @@ struct GModel {
     DevBuf b3;
     DevBuf w3f;                // fp32 [9][128] tap-major weights of the last conv for the fused conv2 epilogue
     bool fuse3 = false;
+    int cta_pairs = 0;         // ctx->cta_pairs at ganrev_load_G: the refinement's backward layers are built with it too
     std::vector<float> blob;   // host copy of the fp32 weight blob: the refinement's backward layers are built from it on first use
 };
 // Noise-vector refinement (ganrev_refine_l2): G's backward layers and the activations one chunk keeps for them.  Built on the
@@ -659,6 +660,7 @@ static int load_G_impl(ganrev_ctx* ctx, int C, int H, int W, int nd, const float
     const float* b3 = p;
 
     G.C = C; G.H = H; G.W = W; G.nd = nd; G.F = F;
+    G.cta_pairs = ctx->cta_pairs;
     const int pairs1 = (ctx->cta_pairs & 1) ? 2 : 1, pairs2 = (ctx->cta_pairs & 2) ? 2 : 1;
     G.kpad = (nd + 63) / 64 * 64;
     {   // Linear + BN1d + ReLU; output features re-ordered from View(512,sH,sW) (NCHW, models.lua:118) to NHWC
@@ -997,7 +999,7 @@ static int build_refine(ganrev_ctx* ctx) {
     const float *g2 = p, *v2 = p + 384; p += 512;
     const float* w3 = p;
     auto sc = [](const float* g, const float* v, size_t i) { return g[i] / std::sqrt(v[i] + 1e-5f); };   // fold_bn's scale
-    const int pairs = (ctx->cta_pairs & 16) ? 2 : 1;   // the pooled 128-wide tile of R conv6 (same kernel shape)
+    const int pairs = (G.cta_pairs & 16) ? 2 : 1;      // the pooled 128-wide tile of R conv6 (same kernel shape); cta_pairs as at load_G
     auto conv_t = [&](TcLayer& L, const char* name, const float* w, const float* g, const float* v, int co_f, int ci_f, int Hin, int Win) {
         // forward conv ci_f -> co_f; adjoint co_f -> ci_f at the forward conv's (high) resolution, pooled to the forward input's
         std::vector<float> wt(static_cast<size_t>(ci_f) * co_f * 9);
@@ -1052,9 +1054,13 @@ static int refine_buffers(ganrev_ctx* ctx, int64_t CH) {
     return GANREV_OK;
 }
 
+// Stages of refine_grad_chunk, in the order it produces them (ganrev_debug_refine_stage numbers them the same way)
+enum { RSTAGE_H0 = 0, RSTAGE_H1, RSTAGE_H2, RSTAGE_Y, RSTAGE_E2, RSTAGE_E1, RSTAGE_E0, RSTAGE_GLIN, RSTAGE_COUNT };
+
 // One forward pass of G keeping h0 / h1 / h2 (bf16 NHWC) and y = G(z) (fp32 NCHW, in R.y), then the backward pass down to
-// R.glin[n x nd] = W_lin^T (s0 e0), the gradient of ||G(z) - x||^2 without the prior term.  n <= CH images.
-static int refine_grad_chunk(ganrev_ctx* ctx, const float* d_z, const float* d_x, int n, int64_t CH) {
+// R.glin[n x nd] = W_lin^T (s0 e0), the gradient of ||G(z) - x||^2 without the prior term.  n <= CH images.  stop_after < RSTAGE_GLIN
+// (tests) returns once that stage's buffer is written: conv1^T writes e0 over e2 in arena[0].
+static int refine_grad_chunk(ganrev_ctx* ctx, const float* d_z, const float* d_x, int n, int64_t CH, int stop_after = RSTAGE_GLIN) {
     GModel& G = ctx->G;
     GRefine& R = ctx->GR;
     const int H = G.H, W = G.W;
@@ -1066,9 +1072,12 @@ static int refine_grad_chunk(ganrev_ctx* ctx, const float* d_z, const float* d_x
         CU_TRY(cudaGetLastError());
     }
     RC_TRY(run_layer(ctx, G.lin, ctx->noise_bf16.p, R.h0.p, n, CH));
+    if (stop_after == RSTAGE_H0) return GANREV_OK;
     RC_TRY(run_layer(ctx, G.c1, R.h0.p, R.h1.p, n, CH));
+    if (stop_after == RSTAGE_H1) return GANREV_OK;
     G.c2.g.w3 = nullptr;                                                        // unfused: h2 itself is needed
     RC_TRY(run_layer(ctx, G.c2, R.h1.p, R.h2.p, n, CH));
+    if (stop_after == RSTAGE_H2) return GANREV_OK;
     G.c3.g.out_sN = 1; G.c3.g.out_sP = 1; G.c3.g.out_sC = static_cast<int>(plane);
     G.c3.bytes_per_img = 2.0 * 128 + 4.0 * 9 * G.C;
     RC_TRY(run_layer(ctx, G.c3, R.h2.p, ctx->arena[1].p, static_cast<int>(npix), CH * H * W));
@@ -1081,6 +1090,7 @@ static int refine_grad_chunk(ganrev_ctx* ctx, const float* d_z, const float* d_x
         else          g_conv3_gather_kernel<3><<<blocks, 256, 0, ctx->stream>>>(planes, plane, static_cast<const float*>(G.b3.p), y, H, W, ilog2(H), ilog2(W), n);
         CU_TRY(cudaGetLastError());
     }
+    if (stop_after == RSTAGE_Y) return GANREV_OK;
     bf16* e2 = static_cast<bf16*>(ctx->arena[0].p);
     {   // per pixel: 9*C taps into 128 channels; reads y, x (9*C neighbours, cached) and h2, writes e2
         ProfScope ps(ctx, "g_bwd_conv3", 2.0 * npix * 9 * G.C * 128, npix * (2.0 * 4 * G.C + 2.0 * 128 + 2.0 * 128));
@@ -1091,10 +1101,13 @@ static int refine_grad_chunk(ganrev_ctx* ctx, const float* d_z, const float* d_x
         else          g_conv3_adjoint_kernel<3><<<blocks, 256, 0, ctx->stream>>>(y, d_x, w3t, h2, e2, H, W, ilog2(H), ilog2(W), n);
         CU_TRY(cudaGetLastError());
     }
+    if (stop_after == RSTAGE_E2) return GANREV_OK;
     R.c2t.g.ref = static_cast<const bf16*>(R.h1.p);
     RC_TRY(run_layer(ctx, R.c2t, e2, ctx->arena[1].p, n, CH));                  // e1 = [h1 > 0] * sumpool(conv2^T(e2))
+    if (stop_after == RSTAGE_E1) return GANREV_OK;
     R.c1t.g.ref = static_cast<const bf16*>(R.h0.p);
     RC_TRY(run_layer(ctx, R.c1t, ctx->arena[1].p, ctx->arena[0].p, n, CH));     // e0 = [h0 > 0] * sumpool(conv1^T(e1))
+    if (stop_after == RSTAGE_E0) return GANREV_OK;
     RC_TRY(run_layer(ctx, R.lint, ctx->arena[0].p, R.glin.p, n, CH));           // W_lin^T (s0 e0)
     return GANREV_OK;
 }
@@ -1489,6 +1502,38 @@ int ganrev_debug_refine_grad(ganrev_ctx* ctx, const float* images, const float* 
         f[i] = dist[i] * dist[i] + static_cast<double>(prior) * zz;
     }
     return GANREV_OK;
+}
+
+int ganrev_debug_refine_stage(ganrev_ctx* ctx, const float* images, const float* z, int64_t N, int stage, void* out, size_t out_bytes) {
+    if (!ctx || !images || !z || !out || N < 0 || stage < 0 || stage >= RSTAGE_COUNT)
+        return ctx ? fail(ctx, GANREV_EINVAL, "bad debug_refine_stage arguments (stage %d)", stage) : GANREV_EINVAL;
+    RC_TRY(refine_check(ctx));
+    const GModel& G = ctx->G;
+    GRefine& R = ctx->GR;
+    const size_t px = static_cast<size_t>(G.H) * G.W;
+    const size_t row[RSTAGE_COUNT] = {static_cast<size_t>(G.F) * 2, px / 4 * 256 * 2, px * 128 * 2, static_cast<size_t>(G.C) * px * 4,
+                                      px * 128 * 2, px / 4 * 256 * 2, static_cast<size_t>(G.F) * 2, static_cast<size_t>(G.nd) * 4};
+    if (out_bytes != row[stage] * static_cast<size_t>(N))
+        return fail(ctx, GANREV_EINVAL, "debug_refine_stage: out_bytes %zu, stage %d of %lld rows needs %zu", out_bytes, stage, (long long)N, row[stage] * static_cast<size_t>(N));
+    if (N == 0) return GANREV_OK;
+    CU_TRY(cudaSetDevice(ctx->device));
+    const int64_t CH = std::min<int64_t>(chunk_for(ctx, G.H, G.W), N);
+    const long long pxc = static_cast<long long>(G.C) * px, nz = N * G.nd;
+    RC_TRY(build_refine(ctx));
+    RC_TRY(refine_buffers(ctx, CH));
+    RC_TRY(ensure(ctx, ctx->stage_a, sizeof(float) * N * pxc));
+    RC_TRY(ensure(ctx, R.zs, sizeof(float) * nz));
+    const float* d_x = static_cast<const float*>(ctx->stage_a.p);
+    const float* d_z = static_cast<const float*>(R.zs.p);
+    CU_TRY(cudaMemcpyAsync(ctx->stage_a.p, images, sizeof(float) * N * pxc, cudaMemcpyHostToDevice, ctx->stream));
+    CU_TRY(cudaMemcpyAsync(R.zs.p, z, sizeof(float) * nz, cudaMemcpyHostToDevice, ctx->stream));
+    const void* src[RSTAGE_COUNT] = {R.h0.p, R.h1.p, R.h2.p, R.y.p, ctx->arena[0].p, ctx->arena[1].p, ctx->arena[0].p, R.glin.p};
+    for (int64_t n0 = 0; n0 < N; n0 += CH) {   // chunks as ganrev_debug_refine_grad runs them; rows land in input order
+        const int n = static_cast<int>(std::min<int64_t>(CH, N - n0));
+        RC_TRY(refine_grad_chunk(ctx, d_z + n0 * G.nd, d_x + n0 * pxc, n, CH, stage));
+        CU_TRY(cudaMemcpyAsync(static_cast<uint8_t*>(out) + n0 * row[stage], src[stage], row[stage] * n, cudaMemcpyDeviceToHost, ctx->stream));
+    }
+    return finish(ctx);
 }
 
 }  // extern "C"

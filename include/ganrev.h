@@ -195,6 +195,12 @@ int ganrev_refine_l2(ganrev_ctx* ctx, int slot, const float* images, const float
 /* Tests: grad [N x nd] = the gradient of f at z and f [N], one forward + backward (no optimiser step). */
 int ganrev_debug_refine_grad(ganrev_ctx* ctx, const float* images, const float* z, int64_t N, float prior,
                              float* grad, double* f);
+/* Tests: one forward + backward pass of G as ganrev_refine_l2 runs it, stopped after `stage`, whose buffer is copied to out
+ * (rows in input order, every chunk): 0 h0 [N][H/4][W/4][512] bf16, 1 h1 [N][H/2][W/2][256] bf16, 2 h2 [N][H][W][128] bf16,
+ * 3 y [N][C][H][W] f32, 4 e2 [N][H][W][128] bf16, 5 e1 [N][H/2][W/2][256] bf16, 6 e0 [N][H/4][W/4][512] bf16, 7 glin [N][nd] f32
+ * (glin + 2 prior z is ganrev_debug_refine_grad's gradient).  GANREV_EINVAL for another stage or an out_bytes that does not match. */
+int ganrev_debug_refine_stage(ganrev_ctx* ctx, const float* images, const float* z, int64_t N, int stage, void* out,
+                              size_t out_bytes);
 
 /* ---- measurement hooks (bench.py) ----------------------------------------------- */
 void*    ganrev_stream(ganrev_ctx* ctx);                 /* cudaStream_t all work runs on */
@@ -225,7 +231,8 @@ int ganrev_debug_trace_read(ganrev_ctx* ctx, int64_t* out);
 /* Tuning / debugging knobs (exact outputs are unaffected; conv_impl 1 differs within the conv tolerance; dbg invalidates results):
  *   "chunk"     images per pipeline chunk; 0 = default = 8192 32x32 faces' worth of pixels
  *   "conv_impl" 0 = tcgen05 implicit GEMM (default), 1 = plain CUDA-core kernels kept for on-device A/B checks
- *   "cta_pairs" bit mask of the conv layers that run as tcgen05 cta_group::2 CTA pairs (default all; read at ganrev_load_*)
+ *   "cta_pairs" bit mask of the conv layers that run as tcgen05 cta_group::2 CTA pairs (default all; read at ganrev_load_*: bit 4 also
+ *               selects it for the refinement's conv2^T / conv1^T, built later from the value ganrev_load_G saw)
  *   "fuse_conv3" 1 = C == 1: the tap products of G's last conv come out of conv2's epilogue (default), 2 = also C == 3 (measured
  *               slower), 0 = separate 1x1 tensor-core pass over the stored activation; read at ganrev_load_G
  *   "xpose2"    1 = second store-transpose buffer per epilogue warp for G's Linear (default), 2 = every plain bf16 layer, 0 = none;
