@@ -39,6 +39,8 @@ _SIGS = {
     "ganrev_refine_l2": (_i, [_vp, _i, _vp, _vp, _i64, _i, _vp, _vp, _vp, _vp]),
     "ganrev_debug_refine_grad": (_i, [_vp, _vp, _vp, _i64, C.c_float, _vp, _vp]),
     "ganrev_debug_refine_stage": (_i, [_vp, _vp, _vp, _i64, _i, _vp, _sz]),
+    "ganrev_debug_G_stage": (_i, [_vp, _vp, _i64, _i, _vp, _sz]),
+    "ganrev_debug_R_stage": (_i, [_vp, _i, _vp, _vp, _i64, _i, _vp, _sz]),
     "ganrev_train_R_init": (_i, [_vp, _i, _i, _i, _i, _i, _i, _vp, _sz]),
     "ganrev_train_R_step": (_i, [_vp, _vp, _i, _vp, _sz, _vp, _vp]),
     "ganrev_train_R_state": (_i, [_vp, _i, _vp, _sz]),
@@ -261,6 +263,36 @@ class Context:
         shape, dt = shapes.get(s, ((1,), np.uint8))
         out = np.empty((N,) + shape, dt)
         self._chk(lib().ganrev_debug_refine_stage(self._h, _ptr(images), _ptr(z), N, s, _ptr(out), out.nbytes))
+        return out
+
+    G_STAGES = ("lin", "c1", "c2", "taps", "y")
+    R_STAGES = ("c1", "c2", "c3", "c4", "c5", "c6", "l1", "out")
+
+    def debug_G_stage(self, noise, stage):
+        """Tests: the output of one layer of forward_G (ganrev.h), rows in input order.  bf16 stages come back as their uint16 bits,
+        NHWC; taps float32 [N][9C][H][W], y float32 NCHW.  `stage` is an index or a name."""
+        Cc, H, W, nd = self.geom
+        s = self.G_STAGES.index(stage) if isinstance(stage, str) else int(stage)
+        noise = _arr(noise, np.float32)
+        shapes = {0: ((H // 4, W // 4, 512), np.uint16), 1: ((H // 2, W // 2, 256), np.uint16), 2: ((H, W, 128), np.uint16),
+                  3: ((9 * Cc, H, W), np.float32), 4: ((Cc, H, W), np.float32)}
+        shape, dt = shapes.get(s, ((1,), np.uint8))
+        out = np.empty((noise.shape[0],) + shape, dt)
+        self._chk(lib().ganrev_debug_G_stage(self._h, _ptr(noise), noise.shape[0], s, _ptr(out), out.nbytes))
+        return out
+
+    def debug_R_stage(self, slot, images, stage, mask=None):
+        """Tests: the output of one layer of forward_R (ganrev.h), rows in input order: bf16 stages as uint16 bits (NHWC; l1 [N][512]),
+        out float32 [N][nd]."""
+        Cc, H, W, nd = self.geom
+        s = self.R_STAGES.index(stage) if isinstance(stage, str) else int(stage)
+        images, mask = _arr(images, np.float32), _arr(mask, np.uint8)
+        shapes = {0: ((H, W, 64), np.uint16), 1: ((H, W, 64), np.uint16), 2: ((H // 2, W // 2, 64), np.uint16),
+                  3: ((H // 2, W // 2, 128), np.uint16), 4: ((H // 2, W // 2, 128), np.uint16), 5: ((H // 4, W // 4, 128), np.uint16),
+                  6: ((512,), np.uint16), 7: ((nd,), np.float32)}
+        shape, dt = shapes.get(s, ((1,), np.uint8))
+        out = np.empty((images.shape[0],) + shape, dt)
+        self._chk(lib().ganrev_debug_R_stage(self._h, slot, _ptr(images), _ptr(mask), images.shape[0], s, _ptr(out), out.nbytes))
         return out
 
     # ---- R training step (train_r.lua:138-170)

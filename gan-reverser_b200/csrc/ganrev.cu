@@ -862,7 +862,14 @@ static int chunk_io_after(ganrev_ctx* ctx, const ChunkIO* io, int64_t c, int64_t
     return GANREV_OK;
 }
 
-static int forward_G_dev(ganrev_ctx* ctx, const float* d_noise, int64_t N, float* d_images, ChunkIO* io = nullptr) {
+// Layers of forward_G_dev / forward_R_dev, in the order they run (ganrev_debug_G_stage / ganrev_debug_R_stage number them the same
+// way).  GLAYER_C2 is G conv2's activation h2, which only exists when the tap products are not fused into conv2's epilogue.
+enum { GLAYER_LIN = 0, GLAYER_C1, GLAYER_C2, GLAYER_TAPS, GLAYER_Y, GLAYER_COUNT };
+enum { RLAYER_C1 = 0, RLAYER_C2, RLAYER_C3, RLAYER_C4, RLAYER_C5, RLAYER_C6, RLAYER_L1, RLAYER_OUT, RLAYER_COUNT };
+
+// stop_after < GLAYER_Y (tests) returns once that layer's buffer is written; call it with N <= one chunk then, or the next chunk
+// overwrites it.
+static int forward_G_dev(ganrev_ctx* ctx, const float* d_noise, int64_t N, float* d_images, ChunkIO* io = nullptr, int stop_after = GLAYER_Y) {
     GModel& G = ctx->G;
     if (!G.loaded) return fail(ctx, GANREV_ESTATE, "G not loaded");
     const int64_t CH = std::min<int64_t>(chunk_for(ctx, G.H, G.W), std::max<int64_t>(N, 1));
@@ -882,7 +889,9 @@ static int forward_G_dev(ganrev_ctx* ctx, const float* d_noise, int64_t N, float
             CU_TRY(cudaGetLastError());
         }
         RC_TRY(run_layer(ctx, G.lin, ctx->noise_bf16.p, ctx->arena[0].p, n, CH));   // [n][sH][sW][512]
+        if (stop_after == GLAYER_LIN) return GANREV_OK;
         RC_TRY(run_layer(ctx, G.c1, ctx->arena[0].p, ctx->arena[1].p, n, CH));      // [n][2sH][2sW][256]
+        if (stop_after == GLAYER_C1) return GANREV_OK;
         // tap products of the last conv as 9*C planes of `plane` floats, P[tap*C + co][pixel]: stores and the gather's loads
         // are then contiguous per warp, and zero-padded columns are never written
         const long long plane = static_cast<long long>(CH) * G.H * G.W;
@@ -892,6 +901,7 @@ static int forward_G_dev(ganrev_ctx* ctx, const float* d_noise, int64_t N, float
         G.c2.g.taps = static_cast<float*>(ctx->arena[0].p);
         G.c2.g.taps_plane = plane;
         RC_TRY(run_layer(ctx, G.c2, ctx->arena[1].p, ctx->arena[0].p, n, CH));      // [n][H][W][128], or (fused) the tap planes
+        if (stop_after == GLAYER_C2) return GANREV_OK;
         {   // last conv: per-pixel tap products (conv2's epilogue, or a 1x1 GEMM on the tensor cores), then the 3x3 gather + bias + sigmoid
             const long long npix = static_cast<long long>(n) * G.H * G.W;
             const float* planes = static_cast<const float*>(ctx->arena[fused ? 0 : 1].p);
@@ -900,6 +910,7 @@ static int forward_G_dev(ganrev_ctx* ctx, const float* d_noise, int64_t N, float
                 G.c3.bytes_per_img = 2.0 * 128 + 4.0 * 9 * G.C;
                 RC_TRY(run_layer(ctx, G.c3, ctx->arena[0].p, ctx->arena[1].p, static_cast<int>(npix), CH * G.H * G.W));
             }
+            if (stop_after == GLAYER_TAPS) return GANREV_OK;
             ProfScope ps(ctx, "g_conv3_gather", 9.0 * npix * G.C, npix * (4.0 * 9 * G.C + 4.0 * G.C));
             const unsigned blocks = static_cast<unsigned>((npix / 4 + 255) / 256);      // a thread per 4 pixels of a row (W >= 16, a power of two)
             float* o = d_images + n0 * G.C * G.H * G.W;
@@ -912,7 +923,9 @@ static int forward_G_dev(ganrev_ctx* ctx, const float* d_noise, int64_t N, float
     return GANREV_OK;
 }
 
-static int forward_R_dev(ganrev_ctx* ctx, int slot, const float* d_images, const uint8_t* d_mask, int64_t N, float* d_attrs, ChunkIO* io = nullptr) {
+// stop_after < RLAYER_OUT (tests): as forward_G_dev.
+static int forward_R_dev(ganrev_ctx* ctx, int slot, const float* d_images, const uint8_t* d_mask, int64_t N, float* d_attrs, ChunkIO* io = nullptr,
+                         int stop_after = RLAYER_OUT) {
     if (slot < 0 || slot > 1) return fail(ctx, GANREV_EINVAL, "slot must be 0 or 1");
     RModel& R = ctx->R[slot];
     if (!R.loaded) return fail(ctx, GANREV_ESTATE, "R slot %d not loaded", slot);
@@ -958,12 +971,19 @@ static int forward_R_dev(ganrev_ctx* ctx, int slot, const float* d_images, const
                 r_conv1_kernel<3><<<blocks, 128, 0, ctx->stream>>>(in, mk, (const float*)R.c1pack.p, reinterpret_cast<bf16*>(ctx->arena[0].p), R.H, R.W, npix);
             CU_TRY(cudaGetLastError());
         }
+        if (stop_after == RLAYER_C1) return GANREV_OK;
         RC_TRY(run_layer(ctx, R.c2, ctx->arena[0].p, ctx->arena[1].p, n, CH));
+        if (stop_after == RLAYER_C2) return GANREV_OK;
         RC_TRY(run_layer(ctx, R.c3, ctx->arena[1].p, ctx->arena[0].p, n, CH));
+        if (stop_after == RLAYER_C3) return GANREV_OK;
         RC_TRY(run_layer(ctx, R.c4, ctx->arena[0].p, ctx->arena[1].p, n, CH));
+        if (stop_after == RLAYER_C4) return GANREV_OK;
         RC_TRY(run_layer(ctx, R.c5, ctx->arena[1].p, ctx->arena[0].p, n, CH));
+        if (stop_after == RLAYER_C5) return GANREV_OK;
         RC_TRY(run_layer(ctx, R.c6, ctx->arena[0].p, ctx->arena[1].p, n, CH));
+        if (stop_after == RLAYER_C6) return GANREV_OK;
         RC_TRY(run_layer(ctx, R.l1, ctx->arena[1].p, ctx->arena[0].p, n, CH));
+        if (stop_after == RLAYER_L1) return GANREV_OK;
         RC_TRY(run_layer(ctx, R.l2, ctx->arena[0].p, d_attrs + n0 * R.nd, n, CH));
         RC_TRY(chunk_io_after(ctx, io, n0 / CH, n_chunks, n0, n));
     }
@@ -1532,6 +1552,80 @@ int ganrev_debug_refine_stage(ganrev_ctx* ctx, const float* images, const float*
         const int n = static_cast<int>(std::min<int64_t>(CH, N - n0));
         RC_TRY(refine_grad_chunk(ctx, d_z + n0 * G.nd, d_x + n0 * pxc, n, CH, stage));
         CU_TRY(cudaMemcpyAsync(static_cast<uint8_t*>(out) + n0 * row[stage], src[stage], row[stage] * n, cudaMemcpyDeviceToHost, ctx->stream));
+    }
+    return finish(ctx);
+}
+
+// Forward layer hooks: forward_G_dev / forward_R_dev run one chunk at a time (n <= the chunk size forward_G / forward_R use, so every
+// layer sees the shapes it sees there), stopped after `stage`; that layer's buffer is copied out after each chunk, rows in input order.
+int ganrev_debug_G_stage(ganrev_ctx* ctx, const float* noise, int64_t N, int stage, void* out, size_t out_bytes) {
+    if (!ctx || !noise || !out || N < 0 || stage < 0 || stage >= GLAYER_COUNT)
+        return ctx ? fail(ctx, GANREV_EINVAL, "bad debug_G_stage arguments (stage %d)", stage) : GANREV_EINVAL;
+    GModel& G = ctx->G;
+    if (!G.loaded) return fail(ctx, GANREV_ESTATE, "G not loaded");
+    const bool fused = G.fuse3 && ctx->conv_impl == 0;
+    if (stage == GLAYER_C2 && fused) return fail(ctx, GANREV_ESTATE, "debug_G_stage: conv2's activation is never stored when the tap products are fused");
+    const size_t px = static_cast<size_t>(G.H) * G.W;
+    const size_t row[GLAYER_COUNT] = {static_cast<size_t>(G.F) * 2, px / 4 * 256 * 2, px * 128 * 2, 9 * static_cast<size_t>(G.C) * px * 4,
+                                      static_cast<size_t>(G.C) * px * 4};
+    if (out_bytes != row[stage] * static_cast<size_t>(N))
+        return fail(ctx, GANREV_EINVAL, "debug_G_stage: out_bytes %zu, stage %d of %lld rows needs %zu", out_bytes, stage, (long long)N, row[stage] * static_cast<size_t>(N));
+    if (N == 0) return GANREV_OK;
+    CU_TRY(cudaSetDevice(ctx->device));
+    const int64_t CH = std::min<int64_t>(chunk_for(ctx, G.H, G.W), N);
+    RC_TRY(ensure(ctx, ctx->stage_a, sizeof(float) * N * G.nd));
+    RC_TRY(ensure(ctx, ctx->stage_b, sizeof(float) * CH * G.C * px));
+    CU_TRY(cudaMemcpyAsync(ctx->stage_a.p, noise, sizeof(float) * N * G.nd, cudaMemcpyHostToDevice, ctx->stream));
+    const float* d_noise = static_cast<const float*>(ctx->stage_a.p);
+    float* d_img = static_cast<float*>(ctx->stage_b.p);
+    uint8_t* o = static_cast<uint8_t*>(out);
+    for (int64_t n0 = 0; n0 < N; n0 += CH) {
+        const int64_t n = std::min<int64_t>(CH, N - n0);
+        RC_TRY(forward_G_dev(ctx, d_noise + n0 * G.nd, n, d_img, nullptr, stage));
+        if (stage == GLAYER_TAPS) {   // plane k of P[k][pixel] (stride: forward_G_dev's chunk of n images) -> out[image][k][H][W]
+            const float* planes = static_cast<const float*>(ctx->arena[fused ? 0 : 1].p);
+            for (int k = 0; k < 9 * G.C; ++k)
+                CU_TRY(cudaMemcpy2DAsync(o + n0 * row[stage] + k * px * 4, row[stage], planes + k * n * px, px * 4, px * 4, n,
+                                         cudaMemcpyDeviceToHost, ctx->stream));
+        } else {
+            const void* src[GLAYER_COUNT] = {ctx->arena[0].p, ctx->arena[1].p, ctx->arena[0].p, nullptr, d_img};
+            CU_TRY(cudaMemcpyAsync(o + n0 * row[stage], src[stage], row[stage] * n, cudaMemcpyDeviceToHost, ctx->stream));
+        }
+    }
+    return finish(ctx);
+}
+
+int ganrev_debug_R_stage(ganrev_ctx* ctx, int slot, const float* images, const uint8_t* mask, int64_t N, int stage, void* out, size_t out_bytes) {
+    if (!ctx || !images || !out || N < 0 || slot < 0 || slot > 1 || stage < 0 || stage >= RLAYER_COUNT)
+        return ctx ? fail(ctx, GANREV_EINVAL, "bad debug_R_stage arguments (slot %d, stage %d)", slot, stage) : GANREV_EINVAL;
+    RModel& R = ctx->R[slot];
+    if (!R.loaded) return fail(ctx, GANREV_ESTATE, "R slot %d not loaded", slot);
+    const size_t px = static_cast<size_t>(R.H) * R.W, pxc = static_cast<size_t>(R.C) * px;
+    const size_t row[RLAYER_COUNT] = {px * 64 * 2, px * 64 * 2, px / 4 * 64 * 2, px / 4 * 128 * 2, px / 4 * 128 * 2, px / 16 * 128 * 2,
+                                      512 * 2, static_cast<size_t>(R.nd) * 4};
+    if (out_bytes != row[stage] * static_cast<size_t>(N))
+        return fail(ctx, GANREV_EINVAL, "debug_R_stage: out_bytes %zu, stage %d of %lld rows needs %zu", out_bytes, stage, (long long)N, row[stage] * static_cast<size_t>(N));
+    if (N == 0) return GANREV_OK;
+    CU_TRY(cudaSetDevice(ctx->device));
+    const int64_t CH = std::min<int64_t>(chunk_for(ctx, R.H, R.W), N);
+    // stage_a: the images; stage_b: the output vectors of one chunk, then the dropout mask
+    const size_t attr_bytes = sizeof(float) * CH * R.nd;
+    RC_TRY(ensure(ctx, ctx->stage_a, sizeof(float) * N * pxc));
+    RC_TRY(ensure(ctx, ctx->stage_b, attr_bytes + (mask ? N * pxc : 0)));
+    CU_TRY(cudaMemcpyAsync(ctx->stage_a.p, images, sizeof(float) * N * pxc, cudaMemcpyHostToDevice, ctx->stream));
+    const uint8_t* d_mask = nullptr;
+    if (mask) {
+        d_mask = static_cast<const uint8_t*>(ctx->stage_b.p) + attr_bytes;
+        CU_TRY(cudaMemcpyAsync(static_cast<uint8_t*>(ctx->stage_b.p) + attr_bytes, mask, N * pxc, cudaMemcpyHostToDevice, ctx->stream));
+    }
+    const float* d_img = static_cast<const float*>(ctx->stage_a.p);
+    float* d_att = static_cast<float*>(ctx->stage_b.p);
+    for (int64_t n0 = 0; n0 < N; n0 += CH) {
+        const int64_t n = std::min<int64_t>(CH, N - n0);
+        RC_TRY(forward_R_dev(ctx, slot, d_img + n0 * pxc, d_mask ? d_mask + n0 * pxc : nullptr, n, d_att, nullptr, stage));
+        // the layers alternate between the two arenas, conv1 writing arena[0]
+        const void* s = stage == RLAYER_OUT ? static_cast<const void*>(d_att) : ctx->arena[stage & 1].p;
+        CU_TRY(cudaMemcpyAsync(static_cast<uint8_t*>(out) + n0 * row[stage], s, row[stage] * n, cudaMemcpyDeviceToHost, ctx->stream));
     }
     return finish(ctx);
 }

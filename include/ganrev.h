@@ -201,6 +201,15 @@ int ganrev_debug_refine_grad(ganrev_ctx* ctx, const float* images, const float* 
  * (glin + 2 prior z is ganrev_debug_refine_grad's gradient).  GANREV_EINVAL for another stage or an out_bytes that does not match. */
 int ganrev_debug_refine_stage(ganrev_ctx* ctx, const float* images, const float* z, int64_t N, int stage, void* out,
                               size_t out_bytes);
+/* Tests: G's forward pass as ganrev_forward_G runs it, chunk by chunk, stopped after layer `stage`, whose buffer is copied to out
+ * (rows in input order): 0 lin [N][H/4][W/4][512] bf16, 1 c1 [N][H/2][W/2][256] bf16, 2 c2 [N][H][W][128] bf16 (GANREV_ESTATE when
+ * the last conv's tap products are fused into conv2: h2 is never stored then), 3 taps [N][9C][H][W] f32 (plane tap*C + co),
+ * 4 y [N][C][H][W] f32.  GANREV_EINVAL for another stage or an out_bytes that does not match. */
+int ganrev_debug_G_stage(ganrev_ctx* ctx, const float* noise, int64_t N, int stage, void* out, size_t out_bytes);
+/* Tests: the same for R of `slot` (mask as ganrev_forward_R): 0..5 conv1..conv6 bf16 NHWC ([N][H][W][64], [N][H][W][64],
+ * [N][H/2][W/2][64] pooled, [N][H/2][W/2][128], [N][H/2][W/2][128], [N][H/4][W/4][128] pooled), 6 l1 [N][512] bf16, 7 out [N][nd] f32. */
+int ganrev_debug_R_stage(ganrev_ctx* ctx, int slot, const float* images, const uint8_t* mask, int64_t N, int stage, void* out,
+                         size_t out_bytes);
 
 /* ---- measurement hooks (bench.py) ----------------------------------------------- */
 void*    ganrev_stream(ganrev_ctx* ctx);                 /* cudaStream_t all work runs on */
