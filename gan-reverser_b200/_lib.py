@@ -39,6 +39,8 @@ _SIGS = {
     "ganrev_refine_l2": (_i, [_vp, _i, _vp, _vp, _i64, _i, _vp, _vp, _vp, _vp]),
     "ganrev_debug_refine_grad": (_i, [_vp, _vp, _vp, _i64, C.c_float, _vp, _vp]),
     "ganrev_debug_refine_stage": (_i, [_vp, _vp, _vp, _i64, _i, _vp, _sz]),
+    "ganrev_refine_masked_l2": (_i, [_vp, _i, _vp, _vp, _vp, _i64, _i, _vp, _vp, _vp, _vp]),
+    "ganrev_debug_refine_masked_stage": (_i, [_vp, _vp, _vp, _vp, _i64, _i, _vp, _sz]),
     "ganrev_debug_G_stage": (_i, [_vp, _vp, _i64, _i, _vp, _sz]),
     "ganrev_debug_R_stage": (_i, [_vp, _i, _vp, _vp, _i64, _i, _vp, _sz]),
     "ganrev_train_R_init": (_i, [_vp, _i, _i, _i, _i, _i, _i, _vp, _sz]),
@@ -250,19 +252,56 @@ class Context:
 
     REFINE_STAGES = ("h0", "h1", "h2", "y", "e2", "e1", "e0", "glin")
 
-    def debug_refine_stage(self, images, z, stage):
-        """Tests: the buffer of one stage of refine_l2's forward + backward pass of G (ganrev.h), rows in input order.  bf16 stages
-        come back as their uint16 bits, NHWC; y is float32 NCHW, glin float32 [N x nd].  `stage` is an index or a name."""
+    def _refine_stage_out(self, N, stage):
         Cc, H, W, nd = self.geom
         s = self.REFINE_STAGES.index(stage) if isinstance(stage, str) else int(stage)
-        images, z = _arr(images, np.float32), _arr(z, np.float32)
-        N = z.shape[0]
         shapes = {0: ((H // 4, W // 4, 512), np.uint16), 1: ((H // 2, W // 2, 256), np.uint16), 2: ((H, W, 128), np.uint16),
                   3: ((Cc, H, W), np.float32), 4: ((H, W, 128), np.uint16), 5: ((H // 2, W // 2, 256), np.uint16),
                   6: ((H // 4, W // 4, 512), np.uint16), 7: ((nd,), np.float32)}
         shape, dt = shapes.get(s, ((1,), np.uint8))
-        out = np.empty((N,) + shape, dt)
+        return s, np.empty((N,) + shape, dt)
+
+    def debug_refine_stage(self, images, z, stage):
+        """Tests: the buffer of one stage of refine_l2's forward + backward pass of G (ganrev.h), rows in input order.  bf16 stages
+        come back as their uint16 bits, NHWC; y is float32 NCHW, glin float32 [N x nd].  `stage` is an index or a name."""
+        images, z = _arr(images, np.float32), _arr(z, np.float32)
+        N = z.shape[0]
+        s, out = self._refine_stage_out(N, stage)
         self._chk(lib().ganrev_debug_refine_stage(self._h, _ptr(images), _ptr(z), N, s, _ptr(out), out.nbytes))
+        return out
+
+    # ---- face completion (new work: refinement against the known pixels only)
+    def refine_masked_l2(self, slot, images, mask, z0=None, iters=100, N=None, lr=0.01, beta1=0.9, beta2=0.999, eps=1e-8, prior=0.0,
+                         zclamp=0.0, want_attrs=True, want_fixed=True):
+        """refine_l2 on sum over mask = 1 of (G(z) - x)^2 + prior ||z||^2; mask is a uint8 keep-mask shaped like images (1 = keep,
+        R's input-mask convention).  images / mask / z0 = None use the resident IMAGES / MASK / ATTRS_slot rows (then N is required).
+        Returns (z_final, G(z_final), masked l2 = sqrt(sum over mask = 1 of (x - G(z_final))^2), not normalised by the kept count)."""
+        Cc, H, W, nd = self.geom
+        images = _arr(images, np.float32)
+        mask = _arr(mask, np.uint8)
+        z0 = _arr(z0, np.float32)
+        if images is not None:
+            N = images.shape[0]
+            assert images.shape[1:] == (Cc, H, W), images.shape
+        if mask is not None:
+            assert mask.shape == (N, Cc, H, W), mask.shape
+        if z0 is not None:
+            assert z0.shape == (N, nd), z0.shape
+        hy = np.array([lr, beta1, beta2, eps, prior, zclamp], np.float32)
+        attrs = np.empty((N, nd), np.float32) if want_attrs else None
+        fixed = np.empty((N, Cc, H, W), np.float32) if want_fixed else None
+        l2 = np.empty((N,), np.float64)
+        self._chk(lib().ganrev_refine_masked_l2(self._h, slot, _ptr(images), _ptr(mask), _ptr(z0), N, int(iters), _ptr(hy),
+                                                _ptr(attrs), _ptr(fixed), _ptr(l2)))
+        return attrs, fixed, l2
+
+    def debug_refine_masked_stage(self, images, mask, z, stage):
+        """Tests: debug_refine_stage with the masked objective (mask: uint8 keep-mask shaped like images)."""
+        images, mask, z = _arr(images, np.float32), _arr(mask, np.uint8), _arr(z, np.float32)
+        N = z.shape[0]
+        assert mask.size == images.size
+        s, out = self._refine_stage_out(N, stage)
+        self._chk(lib().ganrev_debug_refine_masked_stage(self._h, _ptr(images), _ptr(mask), _ptr(z), N, s, _ptr(out), out.nbytes))
         return out
 
     G_STAGES = ("lin", "c1", "c2", "taps", "y")

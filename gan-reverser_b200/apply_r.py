@@ -96,8 +96,26 @@ def refineAttributes(images, attributes, model_G, nbIterations, lr=0.01, prior=0
                                  lr=lr, prior=prior, zclamp=zclamp)
 
 
+def completeFaces(images, mask, model_R_fixer, model_G, nbIterations, lr=0.01, prior=0.0, zclamp=0.0):
+    """New work: complete faces with missing pixels.  mask is a uint8 keep-mask shaped like images (1 = known pixel, R's input-mask
+    convention); the values of images under mask = 0 are never read into any result, whatever they hold.  R_fixer (loaded in slot 1)
+    reads the damaged faces with the mask, then nbIterations Adam steps per image fit G(z) to the known pixels only
+    (ctx.refine_masked_l2 on the resident buffers fix_l2 left).  Returns a dict: attributes (the refined vectors), fixed = G(refined),
+    l2 = the distance over the known pixels (not normalised by their number) and completed = the known pixels with G's values in
+    the holes."""
+    ctx = model_G.ctx
+    assert model_R_fixer.slot == 1, "completeFaces reads the damaged faces with R_fixer in slot 1"
+    images = np.ascontiguousarray(images, np.float32)
+    mask = np.ascontiguousarray(mask, np.uint8)
+    assert mask.shape == images.shape, (mask.shape, images.shape)
+    N = images.shape[0]
+    ctx.fix_l2(1, images, mask, want_attrs=False, want_fixed=False)
+    attributes, fixed, l2 = ctx.refine_masked_l2(1, None, None, None, iters=nbIterations, N=N, lr=lr, prior=prior, zclamp=zclamp)
+    return {"attributes": attributes, "fixed": fixed, "l2": l2, "completed": np.where(mask != 0, images, fixed)}
+
+
 def main(G=None, R=None, R_fixer=None, writeTo="r_results", seed=1, dimensions=(1, 32, 32), noiseDim=100,
-         noiseMethod="normal", colorSpace="y", nbImages=10000, ctx=None, write=True, refine=0):
+         noiseMethod="normal", colorSpace="y", nbImages=10000, ctx=None, write=True, refine=0, complete=0):
     """apply_r.lua main() (apply_r.lua:59-192) end to end.  `G` / `R` / `R_fixer` are paths of Torch7 `.net`
     checkpoints (read with t7.py, geometry from G's `opt` as at :62-79) or None for seeded random-init
     networks of `dimensions` / `noiseDim`.  Same constants as the reference: 16 variation steps, 10,000
@@ -105,7 +123,9 @@ def main(G=None, R=None, R_fixer=None, writeTo="r_results", seed=1, dimensions=(
     anomaly distances at the 15 % quantile.  Returns a dict of everything computed; with `write`, also
     saves the reference's JPEG files under `writeTo` (present.py).  refine > 0 (new work) also refines the fixer's vectors of the
     first 1024 faces by that many Adam steps through G (refineAttributes) and writes fixed_refined.jpg / anomalies_refined.jpg
-    from them; refine = 0 leaves every output as it was."""
+    from them; refine = 0 leaves every output as it was.  complete > 0 (new work) damages the first 528 faces with two seeded masks
+    (completionMasks), completes them with that many Adam steps (completeFaces) and writes completed.jpg; complete = 0 changes no
+    output."""
     from . import models, present
     from .models import default_context
     ctx = ctx or default_context()
@@ -159,6 +179,13 @@ def main(G=None, R=None, R_fixer=None, writeTo="r_results", seed=1, dimensions=(
         flags_r, thr_r = ctx.anomaly_flags(l2_r, 1024, 512 + 16, 0.15)
         out["refined"] = {"attributes": refined, "fixed": fixed_r[:512 + 16], "flags": flags_r.astype(bool),
                           "similarities": 1.0 - l2_r, "anomalyBelow": thr_r}
+    if complete > 0:
+        nComp = 512 + 16
+        orig = np.asarray(images[:nComp], np.float32)
+        mask = completionMasks(orig.shape, seed=seed)
+        rough = ctx.fix_l2(1, orig, mask, want_attrs=False)[1]                                    # G(R_fixer(x, m)), before refinement
+        res = completeFaces(orig, mask, model_R_fixer, model_G, complete)
+        out["completed"] = dict(res, mask=mask, rough=rough)
     if write:
         out["files"].append(present.save(os.path.join(writeTo, "variations.jpg"),
                                          present.toDisplayTensor(out["variations"], nrow=nbSteps, min=0, max=1.0)))
@@ -173,4 +200,21 @@ def main(G=None, R=None, R_fixer=None, writeTo="r_results", seed=1, dimensions=(
                                              present.toDisplayTensor(r["fixed"], nrow=int(math.floor(math.sqrt(n))), min=0, max=1.0)))
             out["files"].append(present.save(os.path.join(writeTo, "anomalies_refined.jpg"),
                                              present.anomalyGrid(np.asarray(images)[:len(r["flags"])], r["flags"], colorSpace)))
+        if complete > 0:
+            c = out["completed"]
+            orig = np.asarray(images[:len(c["mask"])], np.float32)
+            damaged = np.where(c["mask"] != 0, orig, 0.0).astype(np.float32)
+            out["files"].append(present.save(os.path.join(writeTo, "completed.jpg"), present.completionGrid(
+                [damaged, c["rough"], c["fixed"], c["completed"], orig], colorSpace)))
     return out
+
+
+def completionMasks(shape, seed=1):
+    """The keep-masks of main(complete=...): a centred H/2 x W/2 hole (every channel) for the first half of the rows, 50 % pixel
+    dropout (seeded, per element, R_fixer's training distribution) for the rest.  uint8, 1 = keep."""
+    N, C, H, W = shape
+    mask = np.ones(shape, np.uint8)
+    half = N // 2
+    mask[:half, :, H // 4:H // 4 + H // 2, W // 4:W // 4 + W // 2] = 0
+    mask[half:] = (np.random.default_rng(seed + 100).random((N - half, C, H, W)) >= 0.5).astype(np.uint8)
+    return mask

@@ -990,10 +990,14 @@ static int forward_R_dev(ganrev_ctx* ctx, int slot, const float* d_images, const
     return GANREV_OK;
 }
 
-static int l2_dev(ganrev_ctx* ctx, const float* a, const float* b, int64_t N, int px, double* out) {
-    ProfScope ps(ctx, "l2_pairs", 3.0 * N * px, 8.0 * N * px + 8.0 * N);
+// keep == nullptr: torch.dist; otherwise the masked distance over the pixels with keep != 0 (uint8 [N][px])
+static int l2_dev(ganrev_ctx* ctx, const float* a, const float* b, int64_t N, int px, double* out, const uint8_t* keep = nullptr) {
+    ProfScope ps(ctx, keep ? "l2_pairs_masked" : "l2_pairs", 3.0 * N * px, (keep ? 9.0 : 8.0) * N * px + 8.0 * N);
     const unsigned blocks = static_cast<unsigned>((N * 32 + 255) / 256);
-    if (N > 0) l2_pairs_kernel<<<blocks, 256, 0, ctx->stream>>>(a, b, N, px, out);
+    if (N > 0) {
+        if (keep) l2_pairs_kernel<true><<<blocks, 256, 0, ctx->stream>>>(a, b, N, px, out, keep);
+        else      l2_pairs_kernel<false><<<blocks, 256, 0, ctx->stream>>>(a, b, N, px, out, nullptr);
+    }
     CU_TRY(cudaGetLastError());
     return GANREV_OK;
 }
@@ -1079,8 +1083,10 @@ enum { RSTAGE_H0 = 0, RSTAGE_H1, RSTAGE_H2, RSTAGE_Y, RSTAGE_E2, RSTAGE_E1, RSTA
 
 // One forward pass of G keeping h0 / h1 / h2 (bf16 NHWC) and y = G(z) (fp32 NCHW, in R.y), then the backward pass down to
 // R.glin[n x nd] = W_lin^T (s0 e0), the gradient of ||G(z) - x||^2 without the prior term.  n <= CH images.  stop_after < RSTAGE_GLIN
-// (tests) returns once that stage's buffer is written: conv1^T writes e0 over e2 in arena[0].
-static int refine_grad_chunk(ganrev_ctx* ctx, const float* d_z, const float* d_x, int n, int64_t CH, int stop_after = RSTAGE_GLIN) {
+// (tests) returns once that stage's buffer is written: conv1^T writes e0 over e2 in arena[0].  d_keep (uint8 [n][C][H][W], rows as
+// d_x) selects the masked objective, the sum over the kept pixels only (DESIGN.md section 4.7); nullptr = every pixel.
+static int refine_grad_chunk(ganrev_ctx* ctx, const float* d_z, const float* d_x, const uint8_t* d_keep, int n, int64_t CH,
+                             int stop_after = RSTAGE_GLIN) {
     GModel& G = ctx->G;
     GRefine& R = ctx->GR;
     const int H = G.H, W = G.W;
@@ -1112,13 +1118,20 @@ static int refine_grad_chunk(ganrev_ctx* ctx, const float* d_z, const float* d_x
     }
     if (stop_after == RSTAGE_Y) return GANREV_OK;
     bf16* e2 = static_cast<bf16*>(ctx->arena[0].p);
-    {   // per pixel: 9*C taps into 128 channels; reads y, x (9*C neighbours, cached) and h2, writes e2
-        ProfScope ps(ctx, "g_bwd_conv3", 2.0 * npix * 9 * G.C * 128, npix * (2.0 * 4 * G.C + 2.0 * 128 + 2.0 * 128));
+    {   // per pixel: 9*C taps into 128 channels; reads y, x (9*C neighbours, cached), the keep-mask when masked, and h2, writes e2
+        ProfScope ps(ctx, d_keep ? "g_bwd_conv3_masked" : "g_bwd_conv3", 2.0 * npix * 9 * G.C * 128,
+                     npix * ((d_keep ? 9.0 : 8.0) * G.C + 2.0 * 128 + 2.0 * 128));
         const unsigned blocks = static_cast<unsigned>((npix * 16 + 255) / 256);
         const bf16* h2 = static_cast<const bf16*>(R.h2.p);
         const float* w3t = static_cast<const float*>(R.w3t.p);
-        if (G.C == 1) g_conv3_adjoint_kernel<1><<<blocks, 256, 0, ctx->stream>>>(y, d_x, w3t, h2, e2, H, W, ilog2(H), ilog2(W), n);
-        else          g_conv3_adjoint_kernel<3><<<blocks, 256, 0, ctx->stream>>>(y, d_x, w3t, h2, e2, H, W, ilog2(H), ilog2(W), n);
+        const int lgH = ilog2(H), lgW = ilog2(W);
+        if (d_keep) {
+            if (G.C == 1) g_conv3_adjoint_kernel<1, true><<<blocks, 256, 0, ctx->stream>>>(y, d_x, w3t, h2, e2, H, W, lgH, lgW, n, d_keep);
+            else          g_conv3_adjoint_kernel<3, true><<<blocks, 256, 0, ctx->stream>>>(y, d_x, w3t, h2, e2, H, W, lgH, lgW, n, d_keep);
+        } else {
+            if (G.C == 1) g_conv3_adjoint_kernel<1><<<blocks, 256, 0, ctx->stream>>>(y, d_x, w3t, h2, e2, H, W, lgH, lgW, n, nullptr);
+            else          g_conv3_adjoint_kernel<3><<<blocks, 256, 0, ctx->stream>>>(y, d_x, w3t, h2, e2, H, W, lgH, lgW, n, nullptr);
+        }
         CU_TRY(cudaGetLastError());
     }
     if (stop_after == RSTAGE_E2) return GANREV_OK;
@@ -1133,8 +1146,8 @@ static int refine_grad_chunk(ganrev_ctx* ctx, const float* d_z, const float* d_x
 }
 
 // `iters` Adam steps on every row of d_z [N x nd] (in place).  Chunks run one after another, all iterations of a chunk at a time:
-// nothing mixes images, so results do not depend on the chunk size or on which images share a call.
-static int refine_dev(ganrev_ctx* ctx, const float* d_x, float* d_z, int64_t N, int iters, const float* hyper6) {
+// nothing mixes images, so results do not depend on the chunk size or on which images share a call.  d_keep: as refine_grad_chunk.
+static int refine_dev(ganrev_ctx* ctx, const float* d_x, const uint8_t* d_keep, float* d_z, int64_t N, int iters, const float* hyper6) {
     GModel& G = ctx->G;
     GRefine& R = ctx->GR;
     const int64_t CH = std::min<int64_t>(chunk_for(ctx, G.H, G.W), std::max<int64_t>(N, 1));
@@ -1148,7 +1161,7 @@ static int refine_dev(ganrev_ctx* ctx, const float* d_x, float* d_z, int64_t N, 
         CU_TRY(cudaMemsetAsync(R.m.p, 0, sizeof(float) * ne, ctx->stream));
         CU_TRY(cudaMemsetAsync(R.v.p, 0, sizeof(float) * ne, ctx->stream));
         for (int t = 1; t <= iters; ++t) {
-            RC_TRY(refine_grad_chunk(ctx, z, d_x + n0 * px, n, CH));
+            RC_TRY(refine_grad_chunk(ctx, z, d_x + n0 * px, d_keep ? d_keep + n0 * px : nullptr, n, CH));
             RefineHyper h{};
             h.beta1 = hyper6[1]; h.beta2 = hyper6[2]; h.eps = hyper6[3]; h.prior2 = 2.0f * hyper6[4]; h.zclamp = hyper6[5];
             h.step_size = static_cast<float>(static_cast<double>(hyper6[0]) * std::sqrt(1.0 - std::pow(static_cast<double>(h.beta2), static_cast<double>(t))) /
@@ -1448,15 +1461,22 @@ static int refine_check(ganrev_ctx* ctx) {
     return GANREV_OK;
 }
 
-int ganrev_refine_l2(ganrev_ctx* ctx, int slot, const float* images, const float* z0, int64_t N, int iters, const float* hyper6,
-                     float* attrs, float* fixed, double* l2) {
-    if (!ctx || N < 0 || slot < 0 || slot > 1 || !hyper6) return ctx ? fail(ctx, GANREV_EINVAL, "bad refine_l2 arguments") : GANREV_EINVAL;
+// ganrev_refine_l2 (masked = false) and ganrev_refine_masked_l2 (masked = true: mask NULL = the resident MASK buffer)
+static int refine_l2_impl(ganrev_ctx* ctx, int slot, const float* images, bool masked, const uint8_t* mask, const float* z0, int64_t N,
+                          int iters, const float* hyper6, float* attrs, float* fixed, double* l2) {
+    const char* fn = masked ? "refine_masked_l2" : "refine_l2";
+    if (!ctx || N < 0 || slot < 0 || slot > 1 || !hyper6) return ctx ? fail(ctx, GANREV_EINVAL, "bad %s arguments", fn) : GANREV_EINVAL;
     if (iters < 0 || !(hyper6[0] > 0.0f) || !(hyper6[4] >= 0.0f))
-        return fail(ctx, GANREV_EINVAL, "refine_l2 needs iters >= 0, lr > 0, prior >= 0 (got %d, %g, %g)", iters, hyper6[0], hyper6[4]);
+        return fail(ctx, GANREV_EINVAL, "%s needs iters >= 0, lr > 0, prior >= 0 (got %d, %g, %g)", fn, iters, hyper6[0], hyper6[4]);
     RC_TRY(refine_check(ctx));
     if (N == 0) return GANREV_OK;
     CU_TRY(cudaSetDevice(ctx->device));
     RC_TRY(stage_input(ctx, GANREV_BUF_IMAGES, images, N));
+    const uint8_t* d_keep = nullptr;
+    if (masked) {
+        RC_TRY(stage_input(ctx, GANREV_BUF_MASK, mask, N));
+        d_keep = static_cast<const uint8_t*>(ctx->buf[GANREV_BUF_MASK].p);
+    }
     const int ob = slot == 0 ? GANREV_BUF_ATTRS0 : GANREV_BUF_ATTRS1;
     if (z0) {
         RC_TRY(stage_input(ctx, ob, z0, N));                  // (un-sets a database aliasing ATTRS0)
@@ -1471,16 +1491,27 @@ int ganrev_refine_l2(ganrev_ctx* ctx, int slot, const float* images, const float
     const float* d_img = static_cast<const float*>(ctx->buf[GANREV_BUF_IMAGES].p);
     float* d_att = static_cast<float*>(ctx->buf[ob].p);
     float* d_fix = static_cast<float*>(ctx->buf[GANREV_BUF_FIXED].p);
-    if (iters > 0) RC_TRY(refine_dev(ctx, d_img, d_att, N, iters, hyper6));
-    // fixed / l2 from the same path as ganrev_fix_l2: bit-identical to ganrev_forward_G(z_final) + ganrev_l2
+    if (iters > 0) RC_TRY(refine_dev(ctx, d_img, d_keep, d_att, N, iters, hyper6));
+    // fixed / l2 from the same path as ganrev_fix_l2: bit-identical to ganrev_forward_G(z_final) + ganrev_l2 (masked: the masked
+    // distance, bit-identical to ganrev_l2 of where(m, x, 0), where(m, fixed, 0))
     RC_TRY(forward_G_dev(ctx, d_att, N, d_fix));
     ctx->buf_rows[GANREV_BUF_FIXED] = N;
-    RC_TRY(l2_dev(ctx, d_img, d_fix, N, ctx->G.C * ctx->G.H * ctx->G.W, static_cast<double*>(ctx->l2buf.p)));
+    RC_TRY(l2_dev(ctx, d_img, d_fix, N, ctx->G.C * ctx->G.H * ctx->G.W, static_cast<double*>(ctx->l2buf.p), d_keep));
     ctx->l2_valid = N;
     RC_TRY(fetch_output(ctx, ob, attrs, N));
     RC_TRY(fetch_output(ctx, GANREV_BUF_FIXED, fixed, N));
     if (l2) CU_TRY(cudaMemcpyAsync(l2, ctx->l2buf.p, sizeof(double) * N, cudaMemcpyDeviceToHost, ctx->stream));
     return finish(ctx);
+}
+
+int ganrev_refine_l2(ganrev_ctx* ctx, int slot, const float* images, const float* z0, int64_t N, int iters, const float* hyper6,
+                     float* attrs, float* fixed, double* l2) {
+    return refine_l2_impl(ctx, slot, images, false, nullptr, z0, N, iters, hyper6, attrs, fixed, l2);
+}
+
+int ganrev_refine_masked_l2(ganrev_ctx* ctx, int slot, const float* images, const uint8_t* mask, const float* z0, int64_t N,
+                            int iters, const float* hyper6, float* attrs, float* fixed, double* l2) {
+    return refine_l2_impl(ctx, slot, images, true, mask, z0, N, iters, hyper6, attrs, fixed, l2);
 }
 
 int ganrev_debug_refine_grad(ganrev_ctx* ctx, const float* images, const float* z, int64_t N, float prior, float* grad, double* f) {
@@ -1507,7 +1538,7 @@ int ganrev_debug_refine_grad(ganrev_ctx* ctx, const float* images, const float* 
     for (int64_t n0 = 0; n0 < N; n0 += CH) {
         const int n = static_cast<int>(std::min<int64_t>(CH, N - n0));
         const long long ne = static_cast<long long>(n) * G.nd;
-        RC_TRY(refine_grad_chunk(ctx, d_z + n0 * G.nd, d_x + n0 * px, n, CH));
+        RC_TRY(refine_grad_chunk(ctx, d_z + n0 * G.nd, d_x + n0 * px, nullptr, n, CH));
         refine_grad_kernel<<<static_cast<unsigned>((ne + 255) / 256), 256, 0, ctx->stream>>>(static_cast<const float*>(R.glin.p), d_z + n0 * G.nd, 2.0f * prior, d_g + n0 * G.nd, ne);
         CU_TRY(cudaGetLastError());
         RC_TRY(l2_dev(ctx, d_x + n0 * px, static_cast<const float*>(R.y.p), n, static_cast<int>(px), d_dist + n0));
@@ -1524,9 +1555,11 @@ int ganrev_debug_refine_grad(ganrev_ctx* ctx, const float* images, const float* 
     return GANREV_OK;
 }
 
-int ganrev_debug_refine_stage(ganrev_ctx* ctx, const float* images, const float* z, int64_t N, int stage, void* out, size_t out_bytes) {
-    if (!ctx || !images || !z || !out || N < 0 || stage < 0 || stage >= RSTAGE_COUNT)
-        return ctx ? fail(ctx, GANREV_EINVAL, "bad debug_refine_stage arguments (stage %d)", stage) : GANREV_EINVAL;
+// ganrev_debug_refine_stage (masked = false) and ganrev_debug_refine_masked_stage (masked = true, mask required)
+static int debug_refine_stage_impl(ganrev_ctx* ctx, const float* images, bool masked, const uint8_t* mask, const float* z, int64_t N,
+                                   int stage, void* out, size_t out_bytes) {
+    if (!ctx || !images || (masked && !mask) || !z || !out || N < 0 || stage < 0 || stage >= RSTAGE_COUNT)
+        return ctx ? fail(ctx, GANREV_EINVAL, "bad debug_refine_%sstage arguments (stage %d)", masked ? "masked_" : "", stage) : GANREV_EINVAL;
     RC_TRY(refine_check(ctx));
     const GModel& G = ctx->G;
     GRefine& R = ctx->GR;
@@ -1547,13 +1580,28 @@ int ganrev_debug_refine_stage(ganrev_ctx* ctx, const float* images, const float*
     const float* d_z = static_cast<const float*>(R.zs.p);
     CU_TRY(cudaMemcpyAsync(ctx->stage_a.p, images, sizeof(float) * N * pxc, cudaMemcpyHostToDevice, ctx->stream));
     CU_TRY(cudaMemcpyAsync(R.zs.p, z, sizeof(float) * nz, cudaMemcpyHostToDevice, ctx->stream));
+    const uint8_t* d_keep = nullptr;
+    if (masked) {
+        RC_TRY(ensure(ctx, ctx->stage_b, static_cast<size_t>(N) * pxc));
+        CU_TRY(cudaMemcpyAsync(ctx->stage_b.p, mask, static_cast<size_t>(N) * pxc, cudaMemcpyHostToDevice, ctx->stream));
+        d_keep = static_cast<const uint8_t*>(ctx->stage_b.p);
+    }
     const void* src[RSTAGE_COUNT] = {R.h0.p, R.h1.p, R.h2.p, R.y.p, ctx->arena[0].p, ctx->arena[1].p, ctx->arena[0].p, R.glin.p};
     for (int64_t n0 = 0; n0 < N; n0 += CH) {   // chunks as ganrev_debug_refine_grad runs them; rows land in input order
         const int n = static_cast<int>(std::min<int64_t>(CH, N - n0));
-        RC_TRY(refine_grad_chunk(ctx, d_z + n0 * G.nd, d_x + n0 * pxc, n, CH, stage));
+        RC_TRY(refine_grad_chunk(ctx, d_z + n0 * G.nd, d_x + n0 * pxc, d_keep ? d_keep + n0 * pxc : nullptr, n, CH, stage));
         CU_TRY(cudaMemcpyAsync(static_cast<uint8_t*>(out) + n0 * row[stage], src[stage], row[stage] * n, cudaMemcpyDeviceToHost, ctx->stream));
     }
     return finish(ctx);
+}
+
+int ganrev_debug_refine_stage(ganrev_ctx* ctx, const float* images, const float* z, int64_t N, int stage, void* out, size_t out_bytes) {
+    return debug_refine_stage_impl(ctx, images, false, nullptr, z, N, stage, out, out_bytes);
+}
+
+int ganrev_debug_refine_masked_stage(ganrev_ctx* ctx, const float* images, const uint8_t* mask, const float* z, int64_t N, int stage,
+                                     void* out, size_t out_bytes) {
+    return debug_refine_stage_impl(ctx, images, true, mask, z, N, stage, out, out_bytes);
 }
 
 // Forward layer hooks: forward_G_dev / forward_R_dev run one chunk at a time (n <= the chunk size forward_G / forward_R use, so every

@@ -152,29 +152,46 @@ g_conv3_gather_kernel(const float* __restrict__ P, long long plane, const float*
 // ------------------------------------------------------------------ torch.dist, batched
 // Canonical order (mirrored by oracle orc_l2): element i belongs to lane (i/4)%32, each lane
 // adds its fp32 squares in ascending i into a double, then an xor-butterfly over the lanes.
+// MASKED (the masked refinement's distance, DESIGN.md section 4.7): keep[] is a uint8 [n][px] keep-mask and the difference is
+// keep ? x - y : 0 in the same order, so the result is bit-identical to the unmasked kernel on where(keep, x, 0), where(keep, y, 0)
+// (a +0 square added to the double sum changes no bit) and the values under keep = 0 never matter, even NaN / Inf.
+template <bool MASKED = false>
 __global__ void __launch_bounds__(256)
-l2_pairs_kernel(const float* __restrict__ a, const float* __restrict__ b, long long n, int px, double* __restrict__ l2) {
+l2_pairs_kernel(const float* __restrict__ a, const float* __restrict__ b, long long n, int px, double* __restrict__ l2,
+                const uint8_t* __restrict__ keep) {
     const int lane = threadIdx.x & 31;
     const long long pair = (static_cast<long long>(blockIdx.x) * blockDim.x + threadIdx.x) >> 5;
     if (pair >= n) return;
     const float* x = a + pair * px;
     const float* y = b + pair * px;
+    const uint8_t* k = MASKED ? keep + pair * px : nullptr;
     double s = 0.0;
-    const bool vec = ((px & 3) == 0) && ((reinterpret_cast<uintptr_t>(x) & 15) == 0) && ((reinterpret_cast<uintptr_t>(y) & 15) == 0);
+    bool vec = ((px & 3) == 0) && ((reinterpret_cast<uintptr_t>(x) & 15) == 0) && ((reinterpret_cast<uintptr_t>(y) & 15) == 0);
+    if constexpr (MASKED) vec = vec && ((reinterpret_cast<uintptr_t>(k) & 3) == 0);
     if (vec) {
         const float4* x4 = reinterpret_cast<const float4*>(x);
         const float4* y4 = reinterpret_cast<const float4*>(y);
+        const uchar4* k4 = reinterpret_cast<const uchar4*>(k);
         const int n4 = px >> 2;
         int i = lane;
         // 4 independent 128-bit loads per operand in flight
         for (; i + 96 < n4; i += 128) {
             float4 xa[4], ya[4];
+            uchar4 ka[4];
 #pragma unroll
             for (int u = 0; u < 4; ++u) { xa[u] = __ldcs(x4 + i + 32 * u); ya[u] = __ldcs(y4 + i + 32 * u); }
+            if constexpr (MASKED) {
+#pragma unroll
+                for (int u = 0; u < 4; ++u) ka[u] = __ldcs(k4 + i + 32 * u);
+            }
 #pragma unroll
             for (int u = 0; u < 4; ++u) {
                 float d0 = __fsub_rn(xa[u].x, ya[u].x), d1 = __fsub_rn(xa[u].y, ya[u].y);
                 float d2 = __fsub_rn(xa[u].z, ya[u].z), d3 = __fsub_rn(xa[u].w, ya[u].w);
+                if constexpr (MASKED) {
+                    d0 = ka[u].x != 0 ? d0 : 0.0f; d1 = ka[u].y != 0 ? d1 : 0.0f;
+                    d2 = ka[u].z != 0 ? d2 : 0.0f; d3 = ka[u].w != 0 ? d3 : 0.0f;
+                }
                 s += static_cast<double>(__fmul_rn(d0, d0));
                 s += static_cast<double>(__fmul_rn(d1, d1));
                 s += static_cast<double>(__fmul_rn(d2, d2));
@@ -185,6 +202,11 @@ l2_pairs_kernel(const float* __restrict__ a, const float* __restrict__ b, long l
             const float4 xv = __ldcs(x4 + i), yv = __ldcs(y4 + i);
             float d0 = __fsub_rn(xv.x, yv.x), d1 = __fsub_rn(xv.y, yv.y);
             float d2 = __fsub_rn(xv.z, yv.z), d3 = __fsub_rn(xv.w, yv.w);
+            if constexpr (MASKED) {
+                const uchar4 kv = __ldcs(k4 + i);
+                d0 = kv.x != 0 ? d0 : 0.0f; d1 = kv.y != 0 ? d1 : 0.0f;
+                d2 = kv.z != 0 ? d2 : 0.0f; d3 = kv.w != 0 ? d3 : 0.0f;
+            }
             s += static_cast<double>(__fmul_rn(d0, d0));
             s += static_cast<double>(__fmul_rn(d1, d1));
             s += static_cast<double>(__fmul_rn(d2, d2));
@@ -193,7 +215,8 @@ l2_pairs_kernel(const float* __restrict__ a, const float* __restrict__ b, long l
     } else {
         for (int base = lane * 4; base < px; base += 128)
             for (int j = 0; j < 4 && base + j < px; ++j) {
-                const float d = __fsub_rn(x[base + j], y[base + j]);
+                float d = __fsub_rn(x[base + j], y[base + j]);
+                if constexpr (MASKED) d = k[base + j] != 0 ? d : 0.0f;
                 s += static_cast<double>(__fmul_rn(d, d));
             }
     }

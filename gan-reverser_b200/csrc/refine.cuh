@@ -11,10 +11,13 @@ namespace ganrev {
 // One thread per (pixel, 8 consecutive channels): the 16 threads of a pixel read / write its 256 contiguous bytes of h2 / e2.
 // w3t: fp32 [tap = ky*3 + kx][COUT][128] forward weights.  e3 of the output pixel (oy, ox) = (iy + 1 - ky, ix + 1 - kx) is
 // recomputed from y and x by every thread that needs it (cached loads); taps are added in (ky, kx, co) order -- a fixed order.
-template <int COUT>
+// MASKED (ganrev_refine_masked_l2, DESIGN.md section 4.7): keep[] is the uint8 [N][C][H][W] keep-mask of x; e3 = keep ? e3 : 0 at
+// each neighbour, a select, so a hole's x (even NaN / Inf) never reaches e2 and an all-ones mask gives the unmasked bits.
+template <int COUT, bool MASKED = false>
 __global__ void __launch_bounds__(256)
 g_conv3_adjoint_kernel(const float* __restrict__ y, const float* __restrict__ x, const float* __restrict__ w3t,
-                       const bf16* __restrict__ h2, bf16* __restrict__ e2, int H, int W, int lgH, int lgW, long long n_img) {
+                       const bf16* __restrict__ h2, bf16* __restrict__ e2, int H, int W, int lgH, int lgW, long long n_img,
+                       const uint8_t* __restrict__ keep) {
     __shared__ __align__(16) float ws[9 * COUT * 128];
     for (int i = threadIdx.x; i < 9 * COUT * 128; i += blockDim.x) ws[i] = w3t[i];
     __syncthreads();
@@ -40,7 +43,8 @@ g_conv3_adjoint_kernel(const float* __restrict__ y, const float* __restrict__ x,
             for (int co = 0; co < COUT; ++co) {
                 const long long off = ((n * COUT + co) << (lgH + lgW)) + (static_cast<long long>(oy) << lgW) + ox;
                 const float yv = __ldg(y + off), xv = __ldg(x + off);
-                const float e = __fmul_rn(__fmul_rn(2.0f * (yv - xv), yv), 1.0f - yv);   // d/d(pre-sigmoid) of (y - x)^2
+                float e = __fmul_rn(__fmul_rn(2.0f * (yv - xv), yv), 1.0f - yv);         // d/d(pre-sigmoid) of (y - x)^2
+                if constexpr (MASKED) e = __ldg(keep + off) != 0 ? e : 0.0f;
                 const float4* wr = reinterpret_cast<const float4*>(ws + ((ky * 3 + kx) * COUT + co) * 128 + c0);
                 const float4 wa = wr[0], wb = wr[1];
                 acc[0] += wa.x * e; acc[1] += wa.y * e; acc[2] += wa.z * e; acc[3] += wa.w * e;

@@ -43,7 +43,7 @@ int ganrev_kmeans(ganrev_ctx* ctx, int k, int niter, const float* init_centroids
 int ganrev_assign_cosine_min(ganrev_ctx* ctx, const float* centroids, int k, int32_t* cluster, float* cosv);
 int ganrev_cluster_members(ganrev_ctx* ctx, int k, int m, const float* images, int px, int64_t* member_ids, int32_t* member_counts, float* mean_images);
 int ganrev_refine_l2(ganrev_ctx* ctx, int slot, const float* images, const float* z0, int64_t N, int iters, const float* hyper6, float* attrs, float* fixed, double* l2);
-int ganrev_train_R_init(ganrev_ctx* ctx, int C, int H, int W, int noise_dim, int tanh_out, int fixer, const float* blob, size_t n_floats);
+int ganrev_refine_masked_l2(ganrev_ctx* ctx, int slot, const float* images, const uint8_t* mask, const float* z0, int64_t N, int iters, const float* hyper6, float* attrs, float* fixed, double* l2);int ganrev_train_R_init(ganrev_ctx* ctx, int C, int H, int W, int noise_dim, int tanh_out, int fixer, const float* blob, size_t n_floats);
 int ganrev_train_R_step(ganrev_ctx* ctx, const float* noise, int B, const uint8_t* masks, size_t mask_bytes, const float* hyper7, double* loss2);
 int ganrev_train_R_state(ganrev_ctx* ctx, int what, float* out, size_t n_floats);
 int ganrev_sync(ganrev_ctx* ctx);
@@ -303,6 +303,24 @@ function M.refine_l2(ctx, images, attributes, nbIterations, opt, slot)
     local refined, fixed, l2 = torch.FloatTensor(N, attributes:size(2)), torch.FloatTensor(images:size()), torch.DoubleTensor(N)
     check(ctx, lib.ganrev_refine_l2(ctx, slot or 1, images:data(), attributes:data(), N, nbIterations, hyper:data(),
                                     refined:data(), fixed:data(), l2:data()))
+    return refined, fixed, l2
+end
+
+-- New work: face completion.  The same refinement fitted to the known pixels only: mask = ByteTensor shaped like images, 1 = known
+-- (R's input-mask convention, so the mask given to R_fixer:forward(images, mask) serves here too); the values of images under
+-- mask = 0 never influence a result.  l2 is the distance over the known pixels, not normalised by their number.  attributes = the
+-- starting point (e.g. R_fixer:forward(images, mask)).  The composite is the caller's one line (holes must be finite for cmul):
+--   local m = mask:float(); local completed = torch.cmul(images, m) + torch.cmul(fixed, 1 - m)
+function M.refine_masked_l2(ctx, images, mask, attributes, nbIterations, opt, slot)
+    opt = opt or {}
+    images, attributes = images:float():contiguous(), attributes:float():contiguous()
+    mask = mask:byte():contiguous()
+    assert(mask:nElement() == images:nElement(), 'mask must be shaped like images')
+    local N = images:size(1)
+    local hyper = torch.FloatTensor({opt.lr or 0.01, opt.beta1 or 0.9, opt.beta2 or 0.999, opt.eps or 1e-8, opt.prior or 0, opt.zclamp or 0})
+    local refined, fixed, l2 = torch.FloatTensor(N, attributes:size(2)), torch.FloatTensor(images:size()), torch.DoubleTensor(N)
+    check(ctx, lib.ganrev_refine_masked_l2(ctx, slot or 1, images:data(), mask:data(), attributes:data(), N, nbIterations, hyper:data(),
+                                           refined:data(), fixed:data(), l2:data()))
     return refined, fixed, l2
 end
 

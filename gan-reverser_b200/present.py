@@ -169,6 +169,20 @@ def fixedPairsGrid(images, fixed, colorSpace):
     return toDisplayTensor(pairs, nrow=4, min=0, max=1.0)
 
 
+def completionGrid(columns, colorSpace, perRow=4):
+    """New work (face completion, apply_r.completeFaces): one strip per face with the images of `columns` (a list of N x C x H x W
+    arrays, e.g. damaged input | G(R_fixer(x, m)) | G(z_refined) | composite | original) side by side, on a blue background with
+    1-pixel borders as in fixedPairsGrid, perRow strips per row."""
+    cols = [toRgb(np.asarray(c, np.float32), colorSpace) for c in columns]
+    n, _, h, w = cols[0].shape
+    k = len(cols)
+    strips = np.zeros((n, 3, 1 + h + 1, 1 + k * w + 1), np.float32)
+    strips[:, 2] = 1.0
+    for j, c in enumerate(cols):
+        strips[:, :, 1:1 + h, 1 + j * w:1 + (j + 1) * w] = c
+    return toDisplayTensor(strips, nrow=perRow, min=0, max=1.0)
+
+
 def saveFixedFaces(result, colorSpace, writeTo):
     """fixed_pairs.jpg, fixed_images_<N>_unfixed.jpg, fixed_images_<N>.jpg from fixFaces' result (apply_r.lua:344-351)."""
     orig, fixed_pairs = result["pairs"]

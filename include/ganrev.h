@@ -32,8 +32,9 @@
  *   R (models.lua:409-451): 6 x (Conv, BN) with channels C->64->64->64->128->128->128,
  *                           Linear(128*H/4*W/4 -> 512), BN, Linear(512 -> nd).
  *
- * New work beyond the reference is marked as such: multi-GPU sharding and the refinement of recovered noise
- * vectors by gradient descent through G (ganrev_refine_l2).
+ * New work beyond the reference is marked as such: multi-GPU sharding, the refinement of recovered noise
+ * vectors by gradient descent through G (ganrev_refine_l2) and its masked form for completing faces with
+ * missing pixels (ganrev_refine_masked_l2).
  *
  * One geometry per context: G, R and R_fixer of apply_r.lua share {C, H, W, noiseDim}
  * (apply_r.lua:65-79) and the resident buffers are sized by it.  Loading a model with a
@@ -201,6 +202,22 @@ int ganrev_debug_refine_grad(ganrev_ctx* ctx, const float* images, const float* 
  * (glin + 2 prior z is ganrev_debug_refine_grad's gradient).  GANREV_EINVAL for another stage or an out_bytes that does not match. */
 int ganrev_debug_refine_stage(ganrev_ctx* ctx, const float* images, const float* z, int64_t N, int stage, void* out,
                               size_t out_bytes);
+/* ---- face completion: refinement against the known pixels only (new work) ---------------------------------------
+ * ganrev_refine_l2 with the masked objective: mask [N x C x H x W] uint8 is a keep-mask with the layout and the 1 = keep meaning of
+ * R's input mask, so the mask given to ganrev_fix_l2(slot 1, x, mask) serves here too, and
+ *   f(z) = sum over m = 1 of (G(z) - x_i)^2 + prior * ||z||^2,   l2[i] = sqrt(sum over m = 1 of (x_i - G(z_final))^2).
+ * Values of x where m = 0 never influence any result, even NaN or Inf.  l2 is NOT normalised by the number of kept pixels:
+ * comparing images with different mask densities is the caller's business.  mask NULL = the first N rows of the resident MASK
+ * buffer (GANREV_ESTATE if it holds fewer), so ganrev_fix_l2(1, x, m, ..) followed by ganrev_refine_masked_l2(1, NULL, NULL, NULL,
+ * N, ..) runs on resident buffers only.  Everything else -- arguments, resident buffers, outputs (fixed = G(z_final) bit-identical to
+ * ganrev_forward_G, the masked l2 left on the device for ganrev_anomaly_flags(l2 = NULL), iters = 0 = G(z0) with the masked distance),
+ * error codes, determinism, image sharding without a collective -- is exactly ganrev_refine_l2's. */
+int ganrev_refine_masked_l2(ganrev_ctx* ctx, int slot, const float* images, const uint8_t* mask, const float* z0, int64_t N,
+                            int iters, const float* hyper6, float* attrs, float* fixed, double* l2);
+/* Tests: ganrev_debug_refine_stage with the masked objective (mask required): stages 0-3 are unchanged, 4-7 carry the mask;
+ * glin + 2 prior z is the masked gradient. */
+int ganrev_debug_refine_masked_stage(ganrev_ctx* ctx, const float* images, const uint8_t* mask, const float* z, int64_t N,
+                                     int stage, void* out, size_t out_bytes);
 /* Tests: G's forward pass as ganrev_forward_G runs it, chunk by chunk, stopped after layer `stage`, whose buffer is copied to out
  * (rows in input order): 0 lin [N][H/4][W/4][512] bf16, 1 c1 [N][H/2][W/2][256] bf16, 2 c2 [N][H][W][128] bf16 (GANREV_ESTATE when
  * the last conv's tap products are fused into conv2: h2 is never stored then), 3 taps [N][9C][H][W] f32 (plane tap*C + co),

@@ -6,6 +6,10 @@ x = G(z*) and z0 = z* + 0.5 N(0,1) -- the refinement of a rough guess.  Prints o
 iteration over the time of one forward pass of G on the same faces, per-kernel CUDA-event time and executed TFLOP/s of a separate
 profiled run (5 iterations), a PyTorch-CPU autograd + Adam stand-in on a small sample (thread count stated), and the GPU's name,
 power limit and SM clocks read in the same call.  Needs a B200; there is no CPU path for the measured numbers.
+
+--masked: each workload also runs as face completion (ganrev_refine_masked_l2) with a centred H/2 x W/2 hole in every face, timed
+alternately with the unmasked call in the same process (three pairs, the best of each reported), plus its own profiled run.
+Without the flag the output is unchanged.
 """
 import argparse
 import json
@@ -55,12 +59,22 @@ def cpu_standin(pkg, C, H, W, nd, n, iters):
             "geometry": [C, H, W, nd], "faces": n, "iterations": iters, "image_iterations_per_sec": n * iters / dt}
 
 
+def profiled(ctx, run, iters):
+    ctx.profile_reset(); ctx.profile_enable(True)
+    run()
+    ctx.profile_enable(False)
+    return {k: {"launches": v["launches"], "ms_per_iteration": v["ms"] / iters,
+                "tflops_executed": v["flops"] / max(v["ms"], 1e-9) / 1e9, "gbs": v["bytes"] / max(v["ms"], 1e-9) / 1e6}
+            for k, v in ctx.profile().items()}
+
+
 def main():
     ap = argparse.ArgumentParser()
     ap.add_argument("--gpu", type=int, default=0)
     ap.add_argument("--scale", type=float, default=1.0, help="multiply the face counts (quick runs)")
     ap.add_argument("--cpu-faces", type=int, default=8)
     ap.add_argument("--cpu-iters", type=int, default=2)
+    ap.add_argument("--masked", action="store_true", help="also time the masked refinement (centre hole), alternated with the unmasked")
     a = ap.parse_args()
     pkg = load_package()
     ctx = pkg.Context(a.gpu)
@@ -81,17 +95,32 @@ def main():
         _, _, l2_1 = ctx.refine_l2(1, None, z0, iters=iters, N=N, want_attrs=False, want_fixed=False)
         t_iter = (t_ref - t_fwd) / iters            # the call ends with one forward pass + L2 of z_final
         prof_iters = min(iters, 5)
-        ctx.profile_reset(); ctx.profile_enable(True)
-        ctx.refine_l2(1, None, z0, iters=prof_iters, N=N, want_attrs=False, want_fixed=False)
-        ctx.profile_enable(False)
-        kernels = {k: {"launches": v["launches"], "ms_per_iteration": v["ms"] / prof_iters,
-                       "tflops_executed": v["flops"] / max(v["ms"], 1e-9) / 1e9, "gbs": v["bytes"] / max(v["ms"], 1e-9) / 1e6}
-                   for k, v in ctx.profile().items()}
+        kernels = profiled(ctx, lambda: ctx.refine_l2(1, None, z0, iters=prof_iters, N=N, want_attrs=False, want_fixed=False), prof_iters)
         res["workloads"].append({
             "geometry": [C, H, W, nd], "faces": N, "iterations": iters,
             "image_iterations_per_sec": N * iters / (t_ref - t_fwd), "call_s": t_ref, "forward_s": t_fwd,
             "iteration_over_forward": t_iter / t_fwd, "median_l2_before": float(np.median(l2_0)), "median_l2_after": float(np.median(l2_1)),
             "profiled_iterations": prof_iters, "kernels": kernels})
+        if a.masked:
+            mask = np.ones((N, C, H, W), np.uint8)
+            mask[:, :, H // 4:H // 4 + H // 2, W // 4:W // 4 + W // 2] = 0
+            ctx.buffer_put(pkg._lib.BUF_MASK, mask)
+            unmasked = lambda: ctx.refine_l2(1, None, z0, iters=iters, N=N, want_attrs=False, want_fixed=False)
+            masked = lambda: ctx.refine_masked_l2(1, None, None, z0, iters=iters, N=N, want_attrs=False, want_fixed=False)
+            ctx.refine_masked_l2(1, None, None, z0[:min(N, 4096)], iters=2, N=min(N, 4096), want_attrs=False, want_fixed=False)
+            t_u, t_m = [], []
+            for _ in range(3):
+                t_u.append(timed(ctx, unmasked))
+                t_m.append(timed(ctx, masked))
+            _, _, l2_m = ctx.refine_masked_l2(1, None, None, z0, iters=iters, N=N, want_attrs=False, want_fixed=False)
+            res["workloads"][-1]["masked"] = {
+                "mask": "centred H/2 x W/2 hole", "call_s_unmasked": t_u, "call_s_masked": t_m,
+                "image_iterations_per_sec_unmasked": N * iters / (min(t_u) - t_fwd),
+                "image_iterations_per_sec_masked": N * iters / (min(t_m) - t_fwd),
+                "masked_over_unmasked_time": (min(t_m) - t_fwd) / (min(t_u) - t_fwd),
+                "median_masked_l2_after": float(np.median(l2_m)),
+                "kernels": profiled(ctx, lambda: ctx.refine_masked_l2(1, None, None, z0, iters=prof_iters, N=N, want_attrs=False,
+                                                                      want_fixed=False), prof_iters)}
     res["value"] = res["workloads"][0]["image_iterations_per_sec"]
     res["cpu_standin"] = cpu_standin(pkg, 1, 32, 32, 100, a.cpu_faces, a.cpu_iters)
     res["gpu_after"] = gpu_info(a.gpu)
