@@ -342,8 +342,9 @@ static int build_tc_layer(ganrev_ctx* ctx, TcLayer& L, const LayerDef& d, const 
     g.post_scale = d.post_scale; g.out_fp32 = d.out_fp32;
     g.err_flag = ctx->d_err_flag;
 
-    // ---- M tile and tap groups.  Halo reuse needs a whole 128-pixel tile inside one image.
-    const bool halo = d.kind != KIND_LINEAR && d.Hin * d.Win >= 128 && d.Win >= 8;
+    // ---- M tile and tap groups.  Halo reuse needs a whole 128-pixel tile inside one image: BW = min(Win, 16) columns by
+    // BH = 128 / BW rows, so Hin >= BH too (G conv1's 4 x 64 input at 16 x 256 has 256 pixels but only 4 of the 8 rows).
+    const bool halo = d.kind != KIND_LINEAR && d.Win >= 8 && d.Hin * std::min(d.Win, 16) >= 128;
     int BW, BH, BN;
     if (halo) { BW = std::min(d.Win, 16); BH = 128 / BW; BN = 1; }
     else      { BW = std::min(d.Win, d.pool ? 16 : 128); BH = std::min(d.Hin, 128 / BW); BN = 128 / (BW * BH); }

@@ -13,9 +13,15 @@ from util import assert_bitexact, rel_l2, row_cosine
 pytestmark = pytest.mark.gpu
 
 # test_gpu_refine_stages.py's bounds; p and b over the elements with a non-zero reference (holes make many trivially exact zeros)
-C_BOUND = {"e2": 1e-7, "e1": 2e-7, "e0": 2e-7, "glin": 3e-5}
+C_BOUND = {"e2": 2e-7, "e1": 2e-7, "e0": 2e-7, "glin": 3e-5}
 P_MIN = 0.998
 B_MAX = 0.02
+
+
+def _glin_bound(K):
+    """test_gpu_refine_stages.py's: Linear^T's error grows linearly with K = F."""
+    return max(C_BOUND["glin"], 4e-10 * K)
+
 # test_gpu_refine.py's gradient bounds (C = 1: the forward pass's bf16 rounding moves the exact gradient)
 COS_TOL, REL_TOL = 0.999, 3e-2
 COS_TOL_C1, REL_TOL_C1 = 0.996, 8e-2
@@ -25,7 +31,8 @@ COS_TOL_C1, REL_TOL_C1 = 0.996, 8e-2
 COMPLETE_FACTOR = 23.0
 
 STAGE_GEOMS = [(1, 16, 16, 32, 5), (1, 32, 32, 100, 3), (1, 64, 64, 64, 2), (3, 64, 64, 100, 2), (3, 32, 32, 256, 3),
-               (1, 16, 64, 20, 3), (3, 64, 16, 64, 3)]
+               (1, 16, 64, 20, 3), (3, 64, 16, 64, 3), (1, 128, 128, 32, 2), (3, 256, 256, 32, 2), (1, 16, 256, 32, 3),
+               (1, 32, 32, 300, 3)]
 GID = lambda g: "C%dx%dx%d_nd%d_N%d" % g
 STATS = {}
 
@@ -98,7 +105,7 @@ def _check_bf16(key, name, got_bits, ref, tot, relu):
 
 
 # ---------------------------------------------------------------- 1. an all-ones mask is today's refinement, bit for bit
-@pytest.mark.parametrize("geom", [(1, 32, 32, 100, 5), (3, 64, 64, 64, 3), (1, 16, 64, 20, 4)], ids=GID)
+@pytest.mark.parametrize("geom", [(1, 32, 32, 100, 5), (3, 64, 64, 64, 3), (1, 16, 64, 20, 4), (3, 256, 256, 32, 2)], ids=GID)
 def test_all_ones_mask_is_unmasked(pkg, ctx, geom):
     C, H, W, nd, N = geom
     _load(pkg, ctx, C, H, W, nd)
@@ -141,10 +148,38 @@ def test_masked_stages_match_fp64(pkg, ctx, geom, kind):
     ref, tot = tg.ref_glin(tg.bf16_to_f32(st["e0"]).reshape(N, -1), tg.linear_t_weights(p, H, W, nd))
     got = st["glin"].astype(np.float64)
     c_meas = float(np.max(np.abs(got - ref) / np.maximum(tot, 1e-300)))
-    STATS[(key, "glin")] = dict(c=c_meas)
-    assert (np.abs(got - ref) <= C_BOUND["glin"] * tot).all(), f"{key} glin: worst c {c_meas:.3g}"
+    K = 512 * H * W // 16
+    STATS[(key, "glin")] = dict(c=c_meas, K=K)
+    assert (np.abs(got - ref) <= _glin_bound(K) * tot).all(), f"{key} glin: worst c {c_meas:.3g} at K {K}"
     # the forward half is the unmasked one
     assert_bitexact(st["y"], ctx.debug_refine_stage(x, z, "y"), "y")
+
+
+def test_masked_e2_past_2g(pkg, ctx):
+    """1x256x256 at chunk 264 with a block mask: element indices of h2 / e2 pass 2^31 from image 256 on.  The masked e2 of the first
+    and last row of each chunk, rows 127 / 128 and rows past 2^31 / (128 H W) against fp64, and bit-identical to the same rows run
+    alone.  One stage at a time, selected rows only (a stage of e2 is 4.4 GB)."""
+    C, H, W, nd, N, chunk = 1, 256, 256, 32, 265, 264
+    rows = np.array([0, 127, 128, 256, 263, 264])
+    p = _load(pkg, ctx, C, H, W, nd, chunk=chunk)
+    try:
+        x, z = _inputs(C, H, W, nd, N, seed=42)
+        m = block_mask(N, C, H, W)
+        st = {}
+        for s in ("h2", "y", "e2"):
+            a = ctx.debug_refine_masked_stage(x, m, z, s)
+            st[s] = a[rows].copy()
+            del a
+        xr, zr, mr = x[rows].copy(), z[rows].copy(), m[rows].copy()
+        del x, m
+        ctx.set_option("chunk", 0)
+        for s in ("h2", "y", "e2"):
+            assert_bitexact(ctx.debug_refine_masked_stage(xr, mr, zr, s), st[s], f"{s}: rows {rows.tolist()} alone vs inside a 264-image chunk")
+    finally:
+        ctx.set_option("chunk", 0)
+    m2 = tg.bf16_mask(st["h2"])
+    ref, tot = mg.ref_e2(st["y"], xr, p["c3.w"], m2, mask=mr)
+    _check_bf16("C1x256x256_chunk264_block", "e2", st["e2"], ref, tot, m2)
 
 
 # ---------------------------------------------------------------- 3. end-to-end gradient against fp32 masked autograd
